@@ -6,6 +6,7 @@ reverse-diffusion sampling; ms per denoiser step).
   python bench.py --impl reference --steps K --warmup W    the UNMODIFIED reference's CPU path (oracle/_ref via oracle/ref_harness.py)
                                                             on the host cores; the numpy port if that tree is absent
   python bench.py --mode generation --batch 128            BASELINE.json configs[2] (unconditional generation path)
+  python bench.py --steps K --dump-outputs DIR             also writes what the last timed step computed (dump_outputs)
 
 Workload (config 2 of BASELINE.json): base TransformerNetModel (bert-base encoder, seq_len 2096, hidden_dim 128,
 vocab 729), random-init weights, synthetic ComMU-shaped modification batch, 256 sequences per GPU, DDPM chain of
@@ -266,6 +267,8 @@ def run_ours(args):
     torch.cuda.synchronize()
     sampler.stop_flag = True
     ms_decode = d0.elapsed_time(d1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0], tokens)
     t = torch.tensor([ms_total, ms_decode], device=dev, dtype=torch.float64)
     if world > 1:
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
@@ -276,7 +279,7 @@ def run_ours(args):
     # ---- per-kernel breakdown of one step (CUDA events around every launch), dominant-kernel roofline
     peaks = load_peaks()
     prof = None
-    if not args.full_chain and not args.no_breakdown:
+    if not args.full_chain and not args.no_breakdown and n_total + 4 <= DIFFUSION_STEPS:
         # CUDA events around every launch need the eager loop (the timed region above replays the captured step graph):
         # three more steps of the same chain, averaged, so that one step's clock wobble does not pick the dominant kernel
         saved, diffusion.use_cuda_graph = diffusion.use_cuda_graph, False
@@ -320,7 +323,7 @@ def run_ours(args):
     e2e = None
     if not args.full_chain and not args.no_e2e:
         k_e2e = args.steps
-        strength = k_e2e / DIFFUSION_STEPS
+        strength = (k_e2e + 0.5) / DIFFUSION_STEPS                # int(2000 * strength) == k_e2e (k / 2000 can round below)
         for it in range(2):                                        # first pass = warm-up
             dist.barrier()
             torch.cuda.synchronize()
@@ -363,6 +366,24 @@ def run_ours(args):
                 "cpu_baseline": cpu_baseline, "kernels": breakdown}
         print(json.dumps(line))
     dist.barrier()
+
+
+DUMP_BYTES = 56 << 20                                          # --dump-outputs stays below 64 MB in all
+
+
+def dump_outputs(out_dir, sample, tokens):
+    """`--dump-outputs DIR`: what the timed chain hands its caller after its last step, `sample.npy` (x_t, fp32 [n, L, 128]),
+    and the final decode of it, `tokens.npy` (token ids as fp32 [n, L]), for n sequences drawn with a fixed seed from the
+    batch (all of them when they fit DUMP_BYTES; rank 0's batch under torchrun), so that two builds can be compared output
+    for output."""
+    import numpy as np
+    import torch
+    B, Ls, Ds = sample.shape
+    n = min(B, DUMP_BYTES // (Ls * (Ds + 1) * 4))
+    rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(B, n, replace=False))).to(sample.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "sample.npy"), sample.index_select(0, rows).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "tokens.npy"), tokens.index_select(0, rows).cpu().numpy().astype(np.float32))
 
 
 def sample_generation_steps(model, diffusion, model_emb, cond, k_steps, dev):
@@ -433,7 +454,7 @@ def cpu_baseline_sample(mode):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed chain steps (default 10; not with --full-chain)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=256, help="sequences per GPU")
@@ -453,12 +474,23 @@ def main():
     ap.add_argument("--ffn", type=int, default=0)
     ap.add_argument("--layers", type=int, default=0)
     ap.add_argument("--heads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the chain state x_t and its decoded token ids as DIR/<name>.npy "
+                         "(a fixed seeded sample of the sequences, < 64 MB; rank 0's shard under torchrun)")
     args = ap.parse_args()
     set_model_shape(args)
     if (L, H, F, NL, NH) != (2096, 768, 3072, 12, 12):
         args.no_cpu_baseline = True      # the CPU port sample is sized for the base config only
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
+    if args.full_chain and args.steps is not None:
+        ap.error("--full-chain times the %d - warmup steps left after the warm-up; leave --steps out" % DIFFUSION_STEPS)
+    if args.steps is None:
+        args.steps = 10
+    if args.steps < 1 or (not args.full_chain and args.warmup + args.steps > DIFFUSION_STEPS):
+        ap.error("--steps takes 1 to %d - warmup (%d) chain steps" % (DIFFUSION_STEPS, args.warmup))
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computes")
     try:
         if args.impl == "reference":
             run_reference(args)

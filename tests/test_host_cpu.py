@@ -114,7 +114,8 @@ def test_world_size_2_sharding_gloo(tmp_path):
         "print('rank', rank, 'ok')\n" % ROOT)
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
                         "--master-addr", "127.0.0.1", "--master-port", "29611", str(script)],
-                       capture_output=True, text=True, timeout=300)
+                       capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))       # CPU ranks even where a GPU is present
     assert r.returncode == 0, r.stdout + r.stderr
     assert r.stdout.count("ok") == 2
 
