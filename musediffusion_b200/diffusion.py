@@ -121,12 +121,32 @@ def _capture(dev, fn):
     return graph
 
 
+def _noise_kind(mode, top_p):
+    """(noise kind, top_p of the posterior kernel) of one reverse step: DDPM with top_p > 0 draws truncated noise;
+    ddim_sample ignores top_p (diffusion.py:738)."""
+    if mode == _lib.STEP_DDPM and top_p is not None and top_p > 0:
+        return "truncated", top_p
+    return "randn", 0.0
+
+
+def _collect(steps, only_last):
+    """the list p_sample_loop / ddim_sample_loop return: a copy of every sample (the loops reuse their buffers), or the
+    last sample alone (an empty list for an empty chain)."""
+    final = []
+    for sample, _, _, _ in steps:
+        if only_last:
+            final = [sample]
+        else:
+            final.append(sample.clone())
+    return final
+
+
 class GaussianDiffusion:
     """Sampling utilities with the reference's attribute and method names (diffusion.py:121-901)."""
 
     noise_source = None     # optional callable(shape, kind) -> CUDA float tensor; None = in-kernel Philox
     rounding_trace = None   # optional list: every fused rounding call appends (ids int32 [M], top-2 margin fp32 [M]) clones
-    use_cuda_graph = True   # loops of >= GRAPH_MIN_STEPS steps replay ONE captured CUDA graph of a reverse step (fast path only)
+    use_cuda_graph = True   # loops of >= GRAPH_MIN_STEPS steps replay ONE captured CUDA graph of a reverse step (fused path only)
     GRAPH_MIN_STEPS = 4
     seq_offset = 0          # global index of this rank's first sequence (keeps Philox noise shard-invariant)
 
@@ -227,8 +247,9 @@ class GaussianDiffusion:
         return model(x, self._model_timesteps(t), model_kwargs=model_kwargs if model_kwargs is not None else {})
 
     def _step(self, mode, model, x, t, clip_denoised, denoised_fn, model_kwargs, top_p, mask, x_start, eta,
-              want_aux=True, model_output=None, out=None, out_bf16=None, uniform_t=False, step_counter=None):
-        """Shared body of p_sample / ddim_sample: model call, rounding, fused posterior kernel."""
+              want_aux=True, model_output=None, out_bf16=None, noise=None):
+        """Shared body of p_sample / ddim_sample / the generic loop: model call, rounding, fused posterior kernel.
+        `noise`: the step's noise; None takes it from `noise_source`, or draws it in the kernel when that is None too."""
         self._upload_schedule()
         B = x.shape[0]
         assert t.numel() in (1, B)
@@ -239,13 +260,9 @@ class GaussianDiffusion:
         E = rounding_weight_of(denoised_fn)
         idx = pred = None
         if E is not None:
-            # fused distance contraction + row argmin (rounding.py:21-28); tcgen05 split-bf16 kernel when the embedding
-            # width allows it, fp32 CUDA-core kernel otherwise
+            # fused distance contraction + row argmin on the tensor cores (rounding.py:21-28)
             trace = self.rounding_trace
-            if E.shape[1] % 64 == 0:
-                idx = ops.round_argmin_tc(model_output, ops.split_embedding(E), want_margin=trace is not None)
-            else:
-                idx = ops.round_argmin(model_output, E, want_margin=trace is not None)
+            idx = ops.round_argmin_tc(model_output, ops.split_embedding(E), want_margin=trace is not None)
             if trace is not None:
                 idx, margin = idx
                 trace.append((idx.clone(), margin))
@@ -253,17 +270,14 @@ class GaussianDiffusion:
             pred = denoised_fn(model_output, t if t.numel() == B else t.expand(B))   # arbitrary user callable
         else:
             pred = model_output
-        if mode == _lib.STEP_DDPM:
-            kind, tp = ("truncated", top_p) if (top_p is not None and top_p > 0) else ("randn", 0.0)
-        else:
-            kind, tp = "randn", 0.0                                  # ddim_sample ignores top_p (diffusion.py:738)
-        noise = self._external_noise(x.shape, kind, x.device)
+        kind, tp = _noise_kind(mode, top_p)
+        if noise is None:
+            noise = self._external_noise(x.shape, kind, x.device)
         pred_out = torch.empty_like(x, dtype=torch.float32) if want_aux else None
         mean_out = torch.empty_like(x, dtype=torch.float32) if want_aux else None
         sample = ops.posterior_step(
-            x, t, mode, idx=idx, pred=pred, E=E, noise=noise, seed=self._seed(),
-            step_counter=self._next_counter() if step_counter is None else step_counter, seq_offset=self.seq_offset,
-            mask=mask, x_start=x_start, eta=eta, clip=clip_denoised, top_p=tp, out=out, out_bf16=out_bf16,
+            x, t, mode, idx=idx, pred=pred, E=E, noise=noise, seed=self._seed(), step_counter=self._next_counter(),
+            seq_offset=self.seq_offset, mask=mask, x_start=x_start, eta=eta, clip=clip_denoised, top_p=tp, out_bf16=out_bf16,
             pred_out=pred_out, mean_out=mean_out)
         return sample, pred_out, mean_out
 
@@ -276,26 +290,23 @@ class GaussianDiffusion:
         return (mean, _extract_into_tensor(self.posterior_variance, t, x_t.shape),
                 _extract_into_tensor(self.posterior_log_variance_clipped, t, x_t.shape))
 
+    def _mean_variance(self, mean, pred, t, shape):
+        """p_mean_variance's dict (diffusion.py:343-347), with the fixed-large model variance of schedule index t."""
+        return {"mean": mean, "variance": _extract_into_tensor(self.model_variance, t.long(), shape),
+                "log_variance": _extract_into_tensor(self.model_log_variance, t.long(), shape), "pred_xstart": pred}
+
     def p_mean_variance(self, model, x, t, clip_denoised=True, denoised_fn=None, model_kwargs=None):
         """diffusion.py:280-347: dict(mean, variance, log_variance, pred_xstart)."""
-        zeros = torch.zeros_like(x, dtype=torch.float32)
-        saved, self.noise_source = self.noise_source, (lambda shape, kind: zeros)
-        try:
-            _, pred, mean = self._step(_lib.STEP_DDPM, model, x, t, clip_denoised, denoised_fn, model_kwargs, None,
-                                       None, None, 0.0)
-        finally:
-            self.noise_source = saved
-        return {"mean": mean, "variance": _extract_into_tensor(self.model_variance, t, x.shape),
-                "log_variance": _extract_into_tensor(self.model_log_variance, t, x.shape), "pred_xstart": pred}
+        _, pred, mean = self._step(_lib.STEP_DDPM, model, x, t, clip_denoised, denoised_fn, model_kwargs, None, None, None,
+                                   0.0, noise=torch.zeros_like(x, dtype=torch.float32))
+        return self._mean_variance(mean, pred, t, x.shape)
 
     def p_sample(self, model, x, t, clip_denoised=True, denoised_fn=None, model_kwargs=None, top_p=None, mask=None,
                  x_start=None):
         """diffusion.py:349-404."""
         sample, pred, mean = self._step(_lib.STEP_DDPM, model, x, t, clip_denoised, denoised_fn, model_kwargs, top_p,
                                         mask, x_start, 0.0)
-        out = {"mean": mean, "variance": _extract_into_tensor(self.model_variance, t, x.shape),
-               "log_variance": _extract_into_tensor(self.model_log_variance, t, x.shape), "pred_xstart": pred}
-        return {"sample": sample, "pred_xstart": pred, "greedy_mean": mean, "out": out}
+        return {"sample": sample, "pred_xstart": pred, "greedy_mean": mean, "out": self._mean_variance(mean, pred, t, x.shape)}
 
     def ddim_sample(self, model, x, t, clip_denoised=True, denoised_fn=None, model_kwargs=None, eta=0.0,
                     langevin_fn=None, mask=None, x_start=None):
@@ -326,9 +337,12 @@ class GaussianDiffusion:
 
     def _loop(self, mode, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device, progress, top_p,
               clamp_step, clamp_first, mask, x_start, eta, indices, want_aux):
-        """Generator over steps.  Fast path (our denoiser): no per-step allocation, x ping-pongs between two
-        buffers, the posterior kernel also emits the bf16 operand of the next step's first GEMM, one time-embedding
-        row per step (all sequences share t inside the loops, diffusion.py:516,887)."""
+        """Generator of (sample, pred_xstart, mean, t) per reverse step.  Our denoiser, rounding at every step, in-kernel
+        noise and a [B, L, D] state: the fused step body of `_fused_loop`, replayed as a captured CUDA graph for chains of
+        >= GRAPH_MIN_STEPS steps unless `use_cuda_graph` is off or `ops.profile_step` is timing the launches.  Everything
+        else (arbitrary callables, progressive loops, `noise_source`, `rounding_trace`, clamp gating) runs step by step
+        through `_step`; with our denoiser there the posterior kernel also emits the bf16 operand of the next step's first
+        GEMM, and the batch shares one time-embedding row (all sequences share t inside the loops, diffusion.py:516,887)."""
         if device is None:
             device = next(model.parameters()).device
         assert isinstance(shape, (tuple, list))
@@ -370,43 +384,34 @@ class GaussianDiffusion:
             return (i >= clamp_step) if clamp_first else not (i > clamp_step)
 
         E = rounding_weight_of(denoised_fn)
-        graph_ok = (fast is not None and self.use_cuda_graph and len(idx_list) >= self.GRAPH_MIN_STEPS and not want_aux
-                    and self.noise_source is None and self.rounding_trace is None and ops._PROFILE[0] is None
-                    and E is not None and E.shape[1] % 64 == 0 and all(rounds_at(i) for i in idx_list)
-                    and x.dim() == 3)
-        if graph_ok:
-            yield from self._graph_loop(mode, fast, x, E, t_idx, t_model, indices, clip_denoised, top_p, mask, x_start, eta)
+        if (fast is not None and not want_aux and self.noise_source is None and self.rounding_trace is None and E is not None
+                and all(rounds_at(i) for i in idx_list) and x.dim() == 3):
+            capture = self.use_cuda_graph and len(idx_list) >= self.GRAPH_MIN_STEPS and ops._PROFILE[0] is None
+            yield from self._fused_loop(mode, fast, x, E, t_idx, t_model, indices, clip_denoised, top_p, mask, x_start, eta,
+                                        capture)
             return
-        bufs = [torch.empty(tuple(shape), dtype=torch.float32, device=device) for _ in range(2)] if not want_aux else None
-        xb = [torch.empty(tuple(shape), dtype=torch.bfloat16, device=device) for _ in range(2)] if fast is not None else None
         x_bf16 = None
-        mo_buf = torch.empty(tuple(shape), dtype=torch.float32, device=device) if fast is not None else None
         for k, i in enumerate(indices):
             fn = denoised_fn if rounds_at(i) else None
-            t1 = t_idx[k:k + 1]
-            model_output = None
             if fast is not None:
-                model_output = fast.denoise(x, t_model[k:k + 1], x_bf16=x_bf16, uniform_t=True, out=mo_buf)
-            t_arg = t1 if fast is not None else t_idx[k:k + 1].long().expand(B)
-            sample, pred, mean = self._step(
-                mode, model, x, t_arg, clip_denoised, fn, model_kwargs, top_p, mask, x_start, eta, want_aux=want_aux,
-                model_output=model_output, out=None if bufs is None else bufs[k & 1],
-                out_bf16=None if xb is None else xb[k & 1])
-            x = sample
-            x_bf16 = None if xb is None else xb[k & 1]
-            yield sample, pred, mean, t_arg
+                t_arg = t_idx[k:k + 1]
+                model_output = fast.denoise(x, t_model[k:k + 1], x_bf16=x_bf16, uniform_t=True)
+                x_bf16 = torch.empty_like(x, dtype=torch.bfloat16)
+            else:
+                t_arg, model_output = t_idx[k:k + 1].long().expand(B), None
+            x, pred, mean = self._step(mode, model, x, t_arg, clip_denoised, fn, model_kwargs, top_p, mask, x_start, eta,
+                                       want_aux=want_aux, model_output=model_output, out_bf16=x_bf16)
+            yield x, pred, mean, t_arg
 
-    def _graph_loop(self, mode, fast, x, E, t_idx, t_model, indices, clip_denoised, top_p, mask, x_start, eta):
-        """The same chain with ONE reverse step captured as a CUDA graph and replayed (SURVEY.md section 7 step 7).
-        What changes from step to step lives in device memory: `md_step_advance` (first node of the graph) moves a cursor
-        over the index tables and publishes the schedule index, the denoiser's timestep value and the Philox counter of
-        the step; the posterior kernel reads the counter from there, so the noise is bit-identical to the eager loop.
-        x_t is updated in place (the posterior kernel is elementwise) and its bf16 copy feeds the next step's first GEMM.
-        The first step runs eagerly (one-time set-up: shared-memory attributes, weight pack, tensor maps), the graph is
-        captured from the second one."""
+    def _fused_loop(self, mode, fast, x, E, t_idx, t_model, indices, clip_denoised, top_p, mask, x_start, eta, capture):
+        """The chain as one fixed reverse-step body whose per-step inputs live in device memory: `md_step_advance` moves a
+        cursor over the index tables and publishes the schedule index, the denoiser's timestep value and the Philox
+        counter of the step, which the posterior kernel reads.  x_t is updated in place (the posterior kernel is
+        elementwise) and its bf16 copy feeds the next step's first GEMM.
+        `capture`: the first step runs eagerly (one-time set-up: shared-memory attributes, weight pack, tensor maps), the
+        second is captured as a CUDA graph (SURVEY.md section 7 step 7) and every later step replays it.  Otherwise every
+        step launches the same body directly, so per-launch timings measure the kernels a replay runs."""
         dev = x.device
-        n = t_idx.numel()
-        B = x.shape[0]
         self._upload_schedule()
         x = x.clone()                                   # updated in place: never the caller's tensor
         xb = ops.cast_bf16(x)
@@ -425,10 +430,7 @@ class GaussianDiffusion:
         # clip_denoised after rounding = gathering rows of clamp(E, -1, 1): built once per embedding matrix, not per token and step
         E_step, clip_step = (se.E_clamped, 2) if clip_denoised else (E, 0)
         idx = torch.empty((x.shape[0] * x.shape[1],), dtype=torch.int32, device=dev)
-        if mode == _lib.STEP_DDPM:
-            tp = top_p if (top_p is not None and top_p > 0) else 0.0
-        else:
-            tp = 0.0                                    # ddim_sample ignores top_p (diffusion.py:738)
+        _, tp = _noise_kind(mode, top_p)
 
         def one_step():
             ops.step_advance(cursor, t_idx, t_model, t_cur, tm_cur, ctr_cur, ctr_base)
@@ -445,7 +447,7 @@ class GaussianDiffusion:
 
         graph, nodes = None, 0
         for k, i in enumerate(indices):
-            if k == 0:
+            if k == 0 or not capture:
                 one_step()
             else:
                 if graph is None:
@@ -463,16 +465,9 @@ class GaussianDiffusion:
                       x_start=None, gap=1, eta=0.0, t_enc=None, only_last=False):
         """diffusion.py:406-473.  Returns a list of samples (one element when only_last)."""
         indices = list(range(self.num_timesteps))[::-1][slice(t_enc)]
-        final, last = [], None
-        for last in self._loop(_lib.STEP_DDPM, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device,
-                               progress, top_p, clamp_step, clamp_first, mask, x_start, eta, indices, want_aux=False):
-            if not only_last:
-                final.append(last[0].clone())
-        if only_last:
-            if last is None:
-                return []
-            final.append(last[0])
-        return final
+        return _collect(self._loop(_lib.STEP_DDPM, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device,
+                                   progress, top_p, clamp_step, clamp_first, mask, x_start, eta, indices, want_aux=False),
+                        only_last)
 
     def p_sample_loop_progressive(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None,
                                   model_kwargs=None, device=None, progress=False, top_p=None, clamp_step=None,
@@ -483,25 +478,15 @@ class GaussianDiffusion:
                                                 model_kwargs, device, progress, top_p, clamp_step, clamp_first, mask,
                                                 x_start, eta, indices, want_aux=True):
             yield {"sample": sample, "pred_xstart": pred, "greedy_mean": mean,
-                   "out": {"mean": mean, "pred_xstart": pred,
-                           "variance": _extract_into_tensor(self.model_variance, t.long(), sample.shape),
-                           "log_variance": _extract_into_tensor(self.model_log_variance, t.long(), sample.shape)}}
+                   "out": self._mean_variance(mean, pred, t, sample.shape)}
 
     def ddim_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, model_kwargs=None,
                          device=None, progress=False, top_p=None, clamp_step=None, clamp_first=None, mask=None,
                          x_start=None, gap=1, eta=0.0, t_enc=None, only_last=False):
         """diffusion.py:797-846 (top_p / clamp_step / clamp_first accepted and ignored, like the reference)."""
         indices = list(range(self.num_timesteps))[::-1][::gap][slice(t_enc)]
-        final, last = [], None
-        for last in self._loop(_lib.STEP_DDIM, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device,
-                               progress, None, 0, True, mask, x_start, eta, indices, want_aux=False):
-            if not only_last:
-                final.append(last[0].clone())
-        if only_last:
-            if last is None:
-                return []
-            final.append(last[0])
-        return final
+        return _collect(self._loop(_lib.STEP_DDIM, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device,
+                                   progress, None, 0, True, mask, x_start, eta, indices, want_aux=False), only_last)
 
     def ddim_sample_loop_progressive(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None,
                                      model_kwargs=None, device=None, progress=False, eta=0.0, langevin_fn=None,

@@ -246,13 +246,10 @@ class TransformerNetModel(nn.Module):
     def decode_tokens(self, hidden_repr, want_margin=False):
         """get_logits + argmax(-1) (run/sample.py:219-220) fused into one kernel; logits never reach HBM."""
         pk = self.weight_pack()
-        if pk.E.shape[1] % 64 == 0:
-            if pk.split is None:
-                pk.split = ops.SplitEmbedding(pk.E)
-                pk.logit_cst = pk.split.logit_cst(pk.lm_bias)
-            r = ops.round_argmin_tc(hidden_repr, pk.split, cst=pk.logit_cst, mode=1, want_margin=want_margin)
-        else:
-            r = ops.logits_argmax(hidden_repr, pk.E, pk.lm_bias, want_margin=want_margin)
+        if pk.split is None:
+            pk.split = ops.SplitEmbedding(pk.E)
+            pk.logit_cst = pk.split.logit_cst(pk.lm_bias)
+        r = ops.round_argmin_tc(hidden_repr, pk.split, cst=pk.logit_cst, mode=1, want_margin=want_margin)
         if want_margin:
             return r[0].view(hidden_repr.shape[:-1]).long(), r[1].view(hidden_repr.shape[:-1])
         return r.view(hidden_repr.shape[:-1]).long()

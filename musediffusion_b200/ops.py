@@ -39,14 +39,6 @@ def _stream():
     return torch.cuda.current_stream().cuda_stream
 
 
-def _p(t):
-    if t is None:
-        return None
-    if not t.is_cuda:
-        raise _lib.MuseDiffLibraryError("musediffusion_b200 ops need CUDA tensors (got a %s tensor)" % t.device)
-    return t.data_ptr()
-
-
 def _cu(*tensors):
     """every tensor handed to an op lives on a CUDA device (the ops have no other backend)."""
     for t in tensors:

@@ -19,11 +19,14 @@ from .rounding import denoised_fn_round
 
 
 def build_model_emb(model, device):
-    """run/sample.py:92-101: frozen copy of the word embedding used by the rounding callback."""
+    """run/sample.py:92-101: frozen copy of the word embedding used by the rounding callback.  Its split-bf16 form for the
+    tensor-core rounding is built here, once, so the first sampling call launches the same kernels as every later one."""
     w = model.word_embedding.weight
     emb = torch.nn.Embedding(num_embeddings=w.shape[0], embedding_dim=w.shape[1], padding_idx=0,
                              _weight=w.detach().clone())
-    return emb.eval().requires_grad_(False).to(device)
+    emb = emb.eval().requires_grad_(False).to(device)
+    ops.split_embedding(emb.weight)
+    return emb
 
 
 @torch.no_grad()
