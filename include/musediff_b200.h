@@ -54,6 +54,9 @@ int md_set_schedule(const float* tables, int T, cudaStream_t stream);
 /* ---- elementwise / small kernels ---- */
 /* fp32 -> bf16 cast of the state x_t (A operand of the first Linear).  n elements. */
 int md_cast_f32_bf16(const float* in, void* out_bf16, int64_t n, cudaStream_t stream);
+/* The same for fp32 [rows, D] into bf16 rows of stride ld >= D (the padded width Dp of the tensor-core operands, see
+ * md_embed_split_padded); columns D..ld-1 are not written.  D and ld multiples of 4. */
+int md_cast_f32_bf16_ld(const float* in, void* out_bf16, int64_t rows, int D, int ld, cudaStream_t stream);
 /* Models with hidden_dim == encoder hidden size have no input_up_proj / output_down_proj (models/network.py:67-72, 81-86):
  * md_add_pos_time: out[m, :] = bf16((pos[m % L, :] + x[m, :]) + temb[(m / L) * temb_stride, :])  — the pre-LayerNorm sum of
  *   network.py:146-148 taken from the fp32 state itself (emb_x = x, :143-144);  x fp32 [M, H], pos fp32 [L, H].
@@ -81,6 +84,12 @@ int md_layernorm_bf16(const void* in_bf16, const void* resid_bf16, const float* 
  * row) (MD_EPI_BIAS_POS_TIME).  K, N multiples of 8; A, W, out 16-byte aligned. */
 int md_linear_bf16(const void* A, const void* W, const float* bias, void* out, int M, int N, int K, int epilogue,
                    int out_is_f32, const float* pos, const float* temb, int temb_stride, int L, cudaStream_t stream);
+/* md_linear_bf16 storing only the first out_cols <= N columns: out is [M, out_cols] (row stride out_cols, a multiple of
+ * 4 for fp32 and of 8 for bf16 output); the rest is computed and dropped.  The last Linear of a model whose width D is
+ * zero-padded to Dp writes its D real columns this way.  MD_EPI_BIAS_SPLIT needs out_cols == N. */
+int md_linear_bf16_cols(const void* A, const void* W, const float* bias, void* out, int M, int N, int K, int out_cols,
+                        int epilogue, int out_is_f32, const float* pos, const float* temb, int temb_stride, int L,
+                        cudaStream_t stream);
 /* HF BertSelfAttention without mask (called from network.py:151): qkv bf16 [B*L, 3*NH*DH] laid out
  * [q heads | k heads | v heads] per token, q already scaled by 1/sqrt(DH); out bf16 [B*L, NH*DH] = softmax(qk^T) v.
  * DH must be 64. */
@@ -89,10 +98,11 @@ int md_attention_bf16(const void* qkv, void* out, int B, int L, int NH, int DH, 
 /* ---- rounding / decode ---- */
 /* get_efficient_knn (models/rounding.py:21-28): idx[m] = argmin_v clamp(|E_v|^2 + |x_m|^2 - 2 E_v.x_m, 0),
  * lowest v on ties.  x fp32 [M,D], E fp32 [V,D], idx int32 [M]; margin (optional, fp32 [M]) = second-best minus
- * best distance.  D must be 128. */
+ * best distance.  D must be a multiple of 4. */
 int md_round_argmin(const float* x, const float* E, int32_t* idx, float* margin, int64_t M, int V, int D,
                     cudaStream_t stream);
-/* get_logits + argmax (models/network.py:91-93, run/sample.py:219-220): tok[m] = argmax_v (x_m.E_v + bias_v). */
+/* get_logits + argmax (models/network.py:91-93, run/sample.py:219-220): tok[m] = argmax_v (x_m.E_v + bias_v).
+ * D must be a multiple of 4. */
 int md_logits_argmax(const float* x, const float* E, const float* bias, int32_t* tok, float* margin, int64_t M, int V,
                      int D, cudaStream_t stream);
 
@@ -120,6 +130,14 @@ int md_embed_split(const float* E, int V, int D, void* E2, float* sqnorm, float*
                    cudaStream_t stream);
 int md_round_argmin_tc(const float* x, const void* E2, const float* cst, void* x2_ws, int32_t* idx, float* margin,
                        int64_t M, int V, int D, int mode, cudaStream_t stream);
+/* The two entries above for any D that is a multiple of 4, with the bf16 operands zero-padded to the width Dp (a multiple
+ * of 64, >= D; the package uses D rounded up to 64): E2 = bf16 [Vp, 2Dp] = [Eh | 0 | El | 0], x2_ws = bf16 [M, 2Dp] =
+ * [xh | 0 | xl | 0].  The zero columns leave every dot product and |E_v|^2 unchanged, so ids equal those of the unpadded
+ * contraction.  x, E and E_clamped stay fp32 [., D].  With Dp == D these are md_embed_split / md_round_argmin_tc. */
+int md_embed_split_padded(const float* E, int V, int D, int Dp, void* E2, float* sqnorm, float* E_clamped,
+                          cudaStream_t stream);
+int md_round_argmin_tc_padded(const float* x, const void* E2, const float* cst, void* x2_ws, int32_t* idx, float* margin,
+                              int64_t M, int V, int D, int Dp, int mode, cudaStream_t stream);
 
 /* ---- the fused per-step posterior update ----
  * x_{t-1} from x_t for mode DDPM (p_sample :349-404 with p_mean_variance :311-347, q_posterior_mean :257-278) or
@@ -143,6 +161,14 @@ int md_posterior_step(const float* x_t, const int32_t* idx, const float* pred_in
                       const int32_t* mask, int64_t mask_tok_stride, int64_t mask_d_stride, const float* x_start,
                       float* x_out, void* out_bf16, float* pred_out, float* mean_out, int B, int L, int D, int mode,
                       float eta, int clip, float top_p, const uint64_t* step_counter_dev, cudaStream_t stream);
+/* md_posterior_step with out_bf16 rows of stride bf16_ld >= D (a multiple of 4): the padded first-GEMM operand of a
+ * model whose width is not a multiple of 64.  Columns D..bf16_ld-1 are not written (zero them once).  Noise stays keyed
+ * by the logical index (seq_offset*L + m)*D + d. */
+int md_posterior_step_ld(const float* x_t, const int32_t* idx, const float* pred_in, const float* E, const float* noise,
+                         uint64_t seed, uint64_t step_counter, int64_t seq_offset, const int32_t* t, int t_stride,
+                         const int32_t* mask, int64_t mask_tok_stride, int64_t mask_d_stride, const float* x_start,
+                         float* x_out, void* out_bf16, int bf16_ld, float* pred_out, float* mean_out, int B, int L, int D,
+                         int mode, float eta, int clip, float top_p, const uint64_t* step_counter_dev, cudaStream_t stream);
 /* Loop state on the device, so that ONE captured CUDA graph of a reverse step can be replayed for every index of the
  * loops diffusion.py:508-540 / :878-901 (the reference rebuilds t = th.tensor([i] * B) on the host every iteration):
  * k = *cursor; *t_cur = t_idx[k]; *tm_cur = t_model[k] (the value _WrappedModel feeds the denoiser, :1027-1032);
@@ -158,6 +184,10 @@ int md_xstart_from_eps(const float* x_t, const float* eps, const int32_t* t, int
 int md_q_sample(const float* x0, const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
                 const int32_t* t, int t_stride, const int32_t* mask, int64_t mask_tok_stride, int64_t mask_d_stride,
                 float* out, void* out_bf16, int B, int L, int D, cudaStream_t stream);
+/* md_q_sample with out_bf16 rows of stride bf16_ld >= D, as md_posterior_step_ld. */
+int md_q_sample_ld(const float* x0, const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
+                   const int32_t* t, int t_stride, const int32_t* mask, int64_t mask_tok_stride, int64_t mask_d_stride,
+                   float* out, void* out_bf16, int bf16_ld, int B, int L, int D, cudaStream_t stream);
 /* standard-normal / truncated-normal fill with the same Philox stream (testing + generation init). */
 int md_fill_normal(float* out, int64_t n, uint64_t seed, uint64_t step_counter, int64_t elem_offset, float top_p,
                    cudaStream_t stream);

@@ -18,12 +18,14 @@ c_f = ctypes.c_float
 SIGNATURES = {
     "md_set_schedule": [c_p, c_i, c_p],
     "md_cast_f32_bf16": [c_p, c_p, c_i64, c_p],
+    "md_cast_f32_bf16_ld": [c_p, c_p, c_i64, c_i, c_i, c_p],
     "md_cast_bf16_f32": [c_p, c_p, c_i64, c_p],
     "md_add_pos_time": [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_i64, c_p],
     "md_embed_gather": [c_p, c_p, c_i, c_p, c_i64, c_i, c_i, c_p],
     "md_timestep_mlp": [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_p],
     "md_layernorm_bf16": [c_p, c_p, c_p, c_p, c_f, c_p, c_i64, c_i, c_p],
     "md_linear_bf16": [c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_i, c_i, c_p],
+    "md_linear_bf16_cols": [c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_i, c_i, c_p],
     "md_attention_bf16": [c_p, c_p, c_i, c_i, c_i, c_i, c_p],
     "md_round_argmin": [c_p, c_p, c_p, c_p, c_i64, c_i, c_i, c_p],
     "md_logits_argmax": [c_p, c_p, c_p, c_p, c_p, c_i64, c_i, c_i, c_p],
@@ -32,11 +34,16 @@ SIGNATURES = {
     "md_round_tc_padded_vocab": [c_i],
     "md_embed_split": [c_p, c_i, c_i, c_p, c_p, c_p, c_p],
     "md_round_argmin_tc": [c_p, c_p, c_p, c_p, c_p, c_p, c_i64, c_i, c_i, c_i, c_p],
+    "md_embed_split_padded": [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p],
+    "md_round_argmin_tc_padded": [c_p, c_p, c_p, c_p, c_p, c_p, c_i64, c_i, c_i, c_i, c_i, c_p],
     "md_posterior_step": [c_p, c_p, c_p, c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_p,
                           c_p, c_p, c_i, c_i, c_i, c_i, c_f, c_i, c_f, c_p, c_p],
+    "md_posterior_step_ld": [c_p, c_p, c_p, c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_p,
+                             c_i, c_p, c_p, c_i, c_i, c_i, c_i, c_f, c_i, c_f, c_p, c_p],
     "md_step_advance": [c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_u64, c_p],
     "md_xstart_from_eps": [c_p, c_p, c_p, c_i, c_p, c_i, c_i, c_i, c_p],
     "md_q_sample": [c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_i, c_i, c_i, c_p],
+    "md_q_sample_ld": [c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_i, c_i, c_i, c_i, c_p],
     "md_fill_normal": [c_p, c_i64, c_u64, c_u64, c_i64, c_f, c_p],
     "md_decode_prepare": [c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p],
     "md_merge_and_mask": [c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p],

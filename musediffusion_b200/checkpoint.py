@@ -13,6 +13,8 @@
 
    layout:  b"MDPACK01" | u64 header_len | header JSON (utf-8) | padding to 256 | tensor bytes (each 256-aligned)
    header:  {"format": 1, "config": {...model hyper-parameters...}, "tensors": [{"name", "dtype", "shape", "offset", "nbytes"}]}
+   Tensors keep the reference's shapes at every hidden_dim D: a D that is not a multiple of 64 is zero-padded to the
+   tensor-core width when the pack is loaded (`network.WeightPack`), not in the file, so packs of every width share one format.
 """
 import json
 import math

@@ -227,6 +227,7 @@ struct StepArgs {
     float* mean_out;         // optional: posterior mean ("greedy_mean")
     int64_t seq_offset;
     int B, L, D, vshift;
+    int bf16_ld;             // row stride of out_bf16 (>= D; its columns D..bf16_ld-1 are never written)
     float eta;
     int clip;
     NoiseGen rng;
@@ -362,7 +363,8 @@ __global__ void __launch_bounds__(256) posterior_step_kernel(const StepArgs a) {
             }
             st_stream_f4(a.x_out + off[u], o);
             if (a.out_bf16 != nullptr)
-                *reinterpret_cast<uint2*>(a.out_bf16 + off[u]) = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
+                *reinterpret_cast<uint2*>(a.out_bf16 + tok[u] * (IdxT)a.bf16_ld + (IdxT)dd[u]) =
+                    make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
         }
     }
 }
@@ -464,6 +466,7 @@ struct QSampleArgs {
     __nv_bfloat16* out_bf16;
     int64_t seq_offset;
     int B, L, D, vshift;
+    int bf16_ld;             // row stride of out_bf16
     NoiseGen rng;
     const float* sched_dev;
     int T;
@@ -499,7 +502,7 @@ __global__ void __launch_bounds__(256) q_sample_kernel(const QSampleArgs a) {
         }
         st_stream_f4(a.out + off, o);
         if (a.out_bf16 != nullptr)
-            *reinterpret_cast<uint2*>(a.out_bf16 + off) = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
+            *reinterpret_cast<uint2*>(a.out_bf16 + tok * a.bf16_ld + d) = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
     }
 }
 
@@ -549,6 +552,17 @@ __global__ void __launch_bounds__(256) cast_f32_bf16_kernel(const float* in, __n
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         const float4 v = ld_stream_f4(in + i * 4);
         *reinterpret_cast<uint2*>(out + i * 4) = make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
+    }
+}
+// fp32 [rows, D] -> bf16 rows of stride ld >= D (columns D..ld-1 untouched)
+__global__ void __launch_bounds__(256) cast_f32_bf16_ld_kernel(const float* in, __nv_bfloat16* out, int64_t rows, int D, int ld) {
+    const int vec = D >> 2;
+    const int64_t total = rows * vec;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = i / vec;
+        const int c = (int)(i - r * vec) << 2;
+        const float4 v = ld_stream_f4(in + i * 4);
+        *reinterpret_cast<uint2*>(out + r * ld + c) = make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w));
     }
 }
 template <typename IdT>
@@ -797,6 +811,17 @@ extern "C" __attribute__((visibility("default"))) int md_cast_f32_bf16(const flo
     return check_cuda(cudaGetLastError(), "cast launch");
 }
 
+extern "C" __attribute__((visibility("default"))) int md_cast_f32_bf16_ld(const float* in, void* out, int64_t rows, int D, int ld,
+                                                                        cudaStream_t stream) {
+    if (D <= 0 || D % 4 != 0 || ld < D || ld % 4 != 0) {
+        set_last_error("md_cast_f32_bf16_ld: D=%d must be a positive multiple of 4, ld=%d a multiple of 4 >= D", D, ld);
+        return MD_ERR_ARG;
+    }
+    if (rows == 0) return MD_OK;
+    cast_f32_bf16_ld_kernel<<<ew_grid(rows * (D / 4), 256), 256, 0, stream>>>(in, reinterpret_cast<__nv_bfloat16*>(out), rows, D, ld);
+    return check_cuda(cudaGetLastError(), "cast launch");
+}
+
 extern "C" __attribute__((visibility("default"))) int md_cast_bf16_f32(const void* in, float* out, int64_t n, cudaStream_t stream) {
     if (n % 4 != 0) { set_last_error("md_cast_bf16_f32: n must be a multiple of 4"); return MD_ERR_ARG; }
     if (n == 0) return MD_OK;
@@ -861,14 +886,15 @@ extern "C" __attribute__((visibility("default"))) int md_layernorm_bf16(const vo
     return check_cuda(cudaGetLastError(), "layernorm launch");
 }
 
-extern "C" __attribute__((visibility("default"))) int md_posterior_step(const float* x_t, const int32_t* idx, const float* pred_in, const float* E,
+extern "C" __attribute__((visibility("default"))) int md_posterior_step_ld(const float* x_t, const int32_t* idx, const float* pred_in, const float* E,
                                  const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
                                  const int32_t* t, int t_stride, const int32_t* mask, int64_t mask_tok_stride,
-                                 int64_t mask_d_stride, const float* x_start, float* x_out, void* out_bf16,
+                                 int64_t mask_d_stride, const float* x_start, float* x_out, void* out_bf16, int bf16_ld,
                                  float* pred_out, float* mean_out, int B, int L, int D, int mode, float eta, int clip,
                                  float top_p, const uint64_t* step_counter_dev, cudaStream_t stream) {
     if (sched_state().T == 0) { set_last_error("md_posterior_step: md_set_schedule has not been called on this device"); return MD_ERR_ARG; }
     if (D % 4 != 0) { set_last_error("md_posterior_step: D must be a multiple of 4"); return MD_ERR_ARG; }
+    if (bf16_ld < D || bf16_ld % 4 != 0) { set_last_error("md_posterior_step: bf16_ld=%d must be a multiple of 4 >= D=%d", bf16_ld, D); return MD_ERR_ARG; }
     if ((idx == nullptr) == (pred_in == nullptr)) { set_last_error("md_posterior_step: exactly one of idx / pred_in"); return MD_ERR_ARG; }
     if (idx != nullptr && E == nullptr) { set_last_error("md_posterior_step: idx needs E"); return MD_ERR_ARG; }
     if (clip == 2 && idx == nullptr) { set_last_error("md_posterior_step: clip = 2 (pre-clamped E) needs idx"); return MD_ERR_ARG; }
@@ -882,10 +908,11 @@ extern "C" __attribute__((visibility("default"))) int md_posterior_step(const fl
     a.mask_tok_stride = mask_tok_stride; a.mask_d_stride = mask_d_stride; a.x_start = x_start; a.x_out = x_out;
     a.out_bf16 = reinterpret_cast<__nv_bfloat16*>(out_bf16); a.seq_offset = seq_offset; a.B = B; a.L = L; a.D = D;
     a.eta = eta; a.clip = clip; a.rng.init(seed, step_counter, top_p); a.sched = sched_ref(); a.vshift = vec_shift(D);
+    a.bf16_ld = bf16_ld;
     a.step_dev = reinterpret_cast<const unsigned long long*>(step_counter_dev);
     const int grid = ew_grid(((int64_t)B * L * (D / 4) + kStepUnroll - 1) / kStepUnroll, 256);
     const int nz = (noise != nullptr) ? 0 : (a.rng.central ? 1 : 2);
-    if (D == 128 && (mask == nullptr || mask_d_stride == 0) && (int64_t)B * L < (1 << 24)) {
+    if (D == 128 && bf16_ld == 128 && (mask == nullptr || mask_d_stride == 0) && (int64_t)B * L < (1 << 24)) {
         const int g2 = ew_grid(((int64_t)B * L + kStepUnroll - 1) / kStepUnroll * 32, 256);
 #define MD_LAUNCH_FAST(MODE_, CLIP_)                                                                              \
     do {                                                                                                          \
@@ -898,7 +925,7 @@ extern "C" __attribute__((visibility("default"))) int md_posterior_step(const fl
 #undef MD_LAUNCH_FAST
         return check_cuda(cudaGetLastError(), "posterior_step launch");
     }
-    const bool small = (int64_t)B * L * D + (int64_t)grid * 256 * kStepUnroll * 4 < ((int64_t)1 << 31);
+    const bool small = (int64_t)B * L * bf16_ld + (int64_t)grid * 256 * kStepUnroll * 4 < ((int64_t)1 << 31);
 #define MD_LAUNCH_STEP(MODE_, NZ_)                                                                     \
     do {                                                                                               \
         if (small) posterior_step_kernel<MODE_, NZ_, int32_t><<<grid, 256, 0, stream>>>(a);            \
@@ -913,6 +940,17 @@ extern "C" __attribute__((visibility("default"))) int md_posterior_step(const fl
     return check_cuda(cudaGetLastError(), "posterior_step launch");
 }
 
+extern "C" __attribute__((visibility("default"))) int md_posterior_step(const float* x_t, const int32_t* idx, const float* pred_in, const float* E,
+                                 const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
+                                 const int32_t* t, int t_stride, const int32_t* mask, int64_t mask_tok_stride,
+                                 int64_t mask_d_stride, const float* x_start, float* x_out, void* out_bf16,
+                                 float* pred_out, float* mean_out, int B, int L, int D, int mode, float eta, int clip,
+                                 float top_p, const uint64_t* step_counter_dev, cudaStream_t stream) {
+    return md_posterior_step_ld(x_t, idx, pred_in, E, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask_tok_stride,
+                                mask_d_stride, x_start, x_out, out_bf16, D, pred_out, mean_out, B, L, D, mode, eta, clip, top_p,
+                                step_counter_dev, stream);
+}
+
 extern "C" __attribute__((visibility("default"))) int md_xstart_from_eps(const float* x_t, const float* eps, const int32_t* t, int t_stride, float* out, int B, int L,
                                   int D, cudaStream_t stream) {
     if (sched_state().T == 0) { set_last_error("md_xstart_from_eps: md_set_schedule has not been called on this device"); return MD_ERR_ARG; }
@@ -922,18 +960,27 @@ extern "C" __attribute__((visibility("default"))) int md_xstart_from_eps(const f
     return check_cuda(cudaGetLastError(), "xstart_from_eps launch");
 }
 
-extern "C" __attribute__((visibility("default"))) int md_q_sample(const float* x0, const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
+extern "C" __attribute__((visibility("default"))) int md_q_sample_ld(const float* x0, const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
                            const int32_t* t, int t_stride, const int32_t* mask, int64_t mask_tok_stride,
-                           int64_t mask_d_stride, float* out, void* out_bf16, int B, int L, int D, cudaStream_t stream) {
+                           int64_t mask_d_stride, float* out, void* out_bf16, int bf16_ld, int B, int L, int D, cudaStream_t stream) {
     if (t != nullptr && sched_state().T == 0) { set_last_error("md_q_sample: md_set_schedule has not been called on this device"); return MD_ERR_ARG; }
     if (D % 4 != 0) { set_last_error("md_q_sample: D must be a multiple of 4"); return MD_ERR_ARG; }
+    if (bf16_ld < D || bf16_ld % 4 != 0) { set_last_error("md_q_sample: bf16_ld=%d must be a multiple of 4 >= D=%d", bf16_ld, D); return MD_ERR_ARG; }
     if ((int64_t)B * L == 0) return MD_OK;
     QSampleArgs a;
     a.x0 = x0; a.noise = noise; a.t = t; a.t_stride = t_stride ? 1 : 0; a.mask = mask; a.mask_tok_stride = mask_tok_stride; a.mask_d_stride = mask_d_stride;
     a.out = out; a.out_bf16 = reinterpret_cast<__nv_bfloat16*>(out_bf16); a.seq_offset = seq_offset; a.B = B; a.L = L; a.D = D;
     a.rng.init(seed, step_counter, 0.0f); a.sched_dev = sched_state().dev; a.T = sched_state().T; a.vshift = vec_shift(D);
+    a.bf16_ld = bf16_ld;
     q_sample_kernel<<<ew_grid((int64_t)B * L * (D / 4), 256), 256, 0, stream>>>(a);
     return check_cuda(cudaGetLastError(), "q_sample launch");
+}
+
+extern "C" __attribute__((visibility("default"))) int md_q_sample(const float* x0, const float* noise, uint64_t seed, uint64_t step_counter, int64_t seq_offset,
+                           const int32_t* t, int t_stride, const int32_t* mask, int64_t mask_tok_stride,
+                           int64_t mask_d_stride, float* out, void* out_bf16, int B, int L, int D, cudaStream_t stream) {
+    return md_q_sample_ld(x0, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask_tok_stride, mask_d_stride, out, out_bf16,
+                          D, B, L, D, stream);
 }
 
 extern "C" __attribute__((visibility("default"))) int md_fill_normal(float* out, int64_t n, uint64_t seed, uint64_t step_counter, int64_t elem_offset, float top_p,

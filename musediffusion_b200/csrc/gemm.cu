@@ -33,7 +33,8 @@ struct GemmArgs {
     const float* pos;              // [L, N]   (MD_EPI_BIAS_POS_TIME)
     const float* temb;             // [M / L, N] (row stride temb_stride; 0 = one row shared by all sequences)
     int temb_stride;
-    void* out;                     // bf16 or fp32 [M, N]
+    void* out;                     // bf16 or fp32 [M, store_cols]
+    int store_cols;                // output columns kept (<= N; columns beyond are computed and dropped)
     int debug_skip;                // tuning experiments only: 1 = no TMA store, 2 = no slab write + no store
     int idle_wait;                 // bit 0: producer, bit 1: epilogue, bit 2: MMA warp wait with the try_wait suspend hint
 };
@@ -200,7 +201,7 @@ MD_DEVINL void gemm_body(const CUtensorMap& tmA, const CUtensorMap& tmB, const C
             for (int c = 0; c < kChunks; ++c) {
                 const int col0 = hsel * (BN / 2) + c * kChunkCols;      // column inside the tile
                 const int n = n0 + col0;
-                if (n >= p.N) break;                                     // warp-uniform
+                if (n >= p.store_cols) break;                            // warp-uniform
                 float v[kChunkCols];
                 {
                     uint32_t r[32];
@@ -521,11 +522,16 @@ static int dispatch_epi(int epi, const CUtensorMap& tmA, const CUtensorMap& tmB,
 
 using namespace md;
 
-extern "C" __attribute__((visibility("default"))) int md_linear_bf16(const void* A, const void* W, const float* bias, void* out, int M, int N, int K, int epilogue,
-                              int out_is_f32, const float* pos, const float* temb, int temb_stride, int L,
-                              cudaStream_t stream) {
+extern "C" __attribute__((visibility("default"))) int md_linear_bf16_cols(const void* A, const void* W, const float* bias, void* out, int M, int N, int K,
+                                                                        int out_cols, int epilogue, int out_is_f32, const float* pos,
+                                                                        const float* temb, int temb_stride, int L, cudaStream_t stream) {
     if (M <= 0 || N <= 0 || K <= 0) { set_last_error("md_linear_bf16: empty problem M=%d N=%d K=%d", M, N, K); return MD_ERR_ARG; }
     if (K % 8 != 0 || N % 8 != 0) { set_last_error("md_linear_bf16: K and N must be multiples of 8 (K=%d N=%d)", K, N); return MD_ERR_ARG; }
+    // the output's row stride (out_cols elements) must be a multiple of 16 bytes for the TMA store
+    if (out_cols <= 0 || out_cols > N || out_cols % (out_is_f32 ? 4 : 8) != 0) {
+        set_last_error("md_linear_bf16: out_cols=%d must be <= N=%d and a multiple of %d", out_cols, N, out_is_f32 ? 4 : 8);
+        return MD_ERR_ARG;
+    }
     if (epilogue == MD_EPI_BIAS_POS_TIME && (pos == nullptr || temb == nullptr || L <= 0 || M % L != 0)) {
         set_last_error("md_linear_bf16: pos/time epilogue needs pos, temb and L dividing M");
         return MD_ERR_ARG;
@@ -535,14 +541,16 @@ extern "C" __attribute__((visibility("default"))) int md_linear_bf16(const void*
     static const int use_pair = env_int("MD_GEMM_PAIR", 1);
     const bool split = (epilogue == MD_EPI_BIAS_SPLIT);
     if (split && out_is_f32) { set_last_error("md_linear_bf16: the split epilogue writes bf16 [M, 2N]"); return MD_ERR_ARG; }
+    if (split && out_cols != N) { set_last_error("md_linear_bf16: the split epilogue stores all N columns"); return MD_ERR_ARG; }
     const bool pair = use_pair && N % 256 == 0 && M >= 1024 && !out_is_f32 && !split;
     CUtensorMap tmA, tmB, tmC;
     if (int e = make_tmap_2d(&tmA, A, 0, M, K, K, BM, BK)) return e;
     if (int e = make_tmap_2d(&tmB, W, 0, N, K, K, pair ? 128 : BN, BK)) return e;
-    if (int e = make_tmap_2d(&tmC, out, out_is_f32, M, split ? 2 * N : N, split ? 2 * N : N, 32, 32)) return e;
+    // a tile column beyond out_cols is clipped by the TMA store
+    if (int e = make_tmap_2d(&tmC, out, out_is_f32, M, split ? 2 * N : out_cols, split ? 2 * N : out_cols, 32, 32)) return e;
     GemmArgs a;
     a.M = M; a.N = N; a.K = K; a.L = L > 0 ? L : 1;
-    a.bias = bias; a.pos = pos; a.temb = temb; a.temb_stride = temb_stride; a.out = out;
+    a.bias = bias; a.pos = pos; a.temb = temb; a.temb_stride = temb_stride; a.out = out; a.store_cols = out_cols;
     static const int debug_skip = env_int("MD_GEMM_DEBUG_SKIP", 0), idle_env = env_int("MD_GEMM_IDLE", -1);
     a.debug_skip = debug_skip;
     // sleeping waits (try_wait suspend hint) for the warps that wait long: the TMA producer always, the epilogue warps when the
@@ -553,4 +561,10 @@ extern "C" __attribute__((visibility("default"))) int md_linear_bf16(const void*
                                      : dispatch_epi<256, false>(epilogue, tmA, tmB, tmC, a, stream);
     return out_is_f32 ? dispatch_epi<128, true>(epilogue, tmA, tmB, tmC, a, stream)
                       : dispatch_epi<128, false>(epilogue, tmA, tmB, tmC, a, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int md_linear_bf16(const void* A, const void* W, const float* bias, void* out, int M, int N, int K, int epilogue,
+                              int out_is_f32, const float* pos, const float* temb, int temb_stride, int L,
+                              cudaStream_t stream) {
+    return md_linear_bf16_cols(A, W, bias, out, M, N, K, N, epilogue, out_is_f32, pos, temb, temb_stride, L, stream);
 }

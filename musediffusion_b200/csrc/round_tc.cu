@@ -40,41 +40,46 @@ struct RoundTcArgs {
     float* margin;         // optional [M]
 };
 
-// fp32 [rows, D] -> bf16 [rows, copies * 2D] = copies x [hi | lo] split, one float4 per thread
+// fp32 [rows, D] -> bf16 [rows, copies * 2Dp] = copies x [hi | 0 | lo | 0] split (Dp >= D: half width, zero columns
+// D..Dp-1 so that a contraction over Dp columns equals the one over D), one float4 per thread
 __global__ void __launch_bounds__(256) split_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, int64_t rows,
-                                                         int D, int copies) {
-    const int vec = D >> 2;
+                                                         int D, int Dp, int copies) {
+    const int vec = Dp >> 2;
     const int64_t total = rows * vec;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = i / vec;
         const int c = (int)(i - r * vec) << 2;
-        float4 v;
-        asm volatile("ld.global.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(x + r * D + c));
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (c < D)
+            asm volatile("ld.global.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(x + r * D + c));
         const __nv_bfloat162 h0 = __floats2bfloat162_rn(v.x, v.y), h1 = __floats2bfloat162_rn(v.z, v.w);
         const float2 f0 = __bfloat1622float2(h0), f1 = __bfloat1622float2(h1);
         const __nv_bfloat162 l0 = __floats2bfloat162_rn(v.x - f0.x, v.y - f0.y), l1 = __floats2bfloat162_rn(v.z - f1.x, v.w - f1.y);
         for (int k = 0; k < copies; ++k) {
-            __nv_bfloat16* o = out + (r * copies + k) * 2 * D + c;
+            __nv_bfloat16* o = out + (r * copies + k) * 2 * Dp + c;
             *reinterpret_cast<uint2*>(o) = make_uint2(*reinterpret_cast<const uint32_t*>(&h0), *reinterpret_cast<const uint32_t*>(&h1));
-            *reinterpret_cast<uint2*>(o + D) = make_uint2(*reinterpret_cast<const uint32_t*>(&l0), *reinterpret_cast<const uint32_t*>(&l1));
+            *reinterpret_cast<uint2*>(o + Dp) = make_uint2(*reinterpret_cast<const uint32_t*>(&l0), *reinterpret_cast<const uint32_t*>(&l1));
         }
     }
 }
 
-// E fp32 [V, D] -> E2 bf16 [Vp, 2D] = [hi | lo] (zero rows beyond V), |E_v|^2 (fp32, +inf beyond V) and, optionally, the rows
+// E fp32 [V, D] -> E2 bf16 [Vp, 2Dp] = [hi | 0 | lo | 0] (zero rows beyond V, zero columns D..Dp-1), |E_v|^2 over the D real
+// columns (fp32, +inf beyond V) and, optionally, the rows
 // clamped to [-1, 1] (what clip_denoised makes of a rounded x0, diffusion.py:323-324: the posterior kernel then gathers them
 // ready-made instead of clamping 128 values per token and step)
 __global__ void __launch_bounds__(128) embed_prepare_kernel(const float* __restrict__ E, __nv_bfloat16* __restrict__ E2,
-                                                            float* __restrict__ sqnorm, float* __restrict__ E_clamped, int V, int Vp, int D) {
+                                                            float* __restrict__ sqnorm, float* __restrict__ E_clamped, int V, int Vp, int D,
+                                                            int Dp) {
     const int v = blockIdx.x;
     float s = 0.f;
-    for (int d = threadIdx.x; d < D; d += blockDim.x) {
-        const float e = (v < V) ? E[(size_t)v * D + d] : 0.f;
+    for (int d = threadIdx.x; d < Dp; d += blockDim.x) {
+        const bool real = v < V && d < D;
+        const float e = real ? E[(size_t)v * D + d] : 0.f;
         const __nv_bfloat16 h = __float2bfloat16_rn(e);
-        E2[(size_t)v * 2 * D + d] = h;
-        E2[(size_t)v * 2 * D + D + d] = __float2bfloat16_rn(e - __bfloat162float(h));
-        if (E_clamped != nullptr && v < V) E_clamped[(size_t)v * D + d] = fminf(fmaxf(e, -1.0f), 1.0f);
-        s = fmaf(e, e, s);
+        E2[(size_t)v * 2 * Dp + d] = h;
+        E2[(size_t)v * 2 * Dp + Dp + d] = __float2bfloat16_rn(e - __bfloat162float(h));
+        if (E_clamped != nullptr && real) E_clamped[(size_t)v * D + d] = fminf(fmaxf(e, -1.0f), 1.0f);
+        if (d < D) s = fmaf(e, e, s);
     }
     __shared__ float red[4];
 #pragma unroll
@@ -246,36 +251,52 @@ using namespace md;
 
 extern "C" __attribute__((visibility("default"))) int md_round_tc_padded_vocab(int V) { return (V + RT_BN - 1) / RT_BN * RT_BN; }
 
+static bool padded_width_ok(int D, int Dp) { return D > 0 && D % 4 == 0 && Dp >= D && Dp % RT_BK == 0; }
+
+extern "C" __attribute__((visibility("default"))) int md_embed_split_padded(const float* E, int V, int D, int Dp, void* E2, float* sqnorm,
+                                                                          float* E_clamped, cudaStream_t stream) {
+    if (V <= 0 || !padded_width_ok(D, Dp)) {
+        set_last_error("md_embed_split_padded: D=%d must be a positive multiple of 4, Dp=%d a multiple of %d >= D", D, Dp, RT_BK);
+        return MD_ERR_ARG;
+    }
+    const int Vp = md_round_tc_padded_vocab(V);
+    embed_prepare_kernel<<<Vp, 128, 0, stream>>>(E, reinterpret_cast<__nv_bfloat16*>(E2), sqnorm, E_clamped, V, Vp, D, Dp);
+    return check_cuda(cudaGetLastError(), "embed_split launch");
+}
+
 extern "C" __attribute__((visibility("default"))) int md_embed_split(const float* E, int V, int D, void* E2, float* sqnorm, float* E_clamped, cudaStream_t stream) {
     if (V <= 0 || D <= 0 || D % RT_BK != 0) { set_last_error("md_embed_split: D=%d must be a positive multiple of %d", D, RT_BK); return MD_ERR_ARG; }
-    const int Vp = md_round_tc_padded_vocab(V);
-    embed_prepare_kernel<<<Vp, 128, 0, stream>>>(E, reinterpret_cast<__nv_bfloat16*>(E2), sqnorm, E_clamped, V, Vp, D);
-    return check_cuda(cudaGetLastError(), "embed_split launch");
+    return md_embed_split_padded(E, V, D, D, E2, sqnorm, E_clamped, stream);
 }
 
 extern "C" __attribute__((visibility("default"))) int md_split_bf16(const float* x, void* out, int64_t rows, int D, int copies, cudaStream_t stream) {
     if (D <= 0 || D % 4 != 0 || copies < 1) { set_last_error("md_split_bf16: D=%d must be a positive multiple of 4, copies >= 1", D); return MD_ERR_ARG; }
     if (rows == 0) return MD_OK;
-    split_bf16_kernel<<<ew_grid2(rows * (D / 4)), 256, 0, stream>>>(x, reinterpret_cast<__nv_bfloat16*>(out), rows, D, copies);
+    split_bf16_kernel<<<ew_grid2(rows * (D / 4)), 256, 0, stream>>>(x, reinterpret_cast<__nv_bfloat16*>(out), rows, D, D, copies);
     return check_cuda(cudaGetLastError(), "split_bf16 launch");
 }
 
-extern "C" __attribute__((visibility("default"))) int md_round_argmin_tc(const float* x, const void* E2, const float* cst, void* x2_ws, int32_t* idx, float* margin,
-                                  int64_t M, int V, int D, int mode, cudaStream_t stream) {
-    if (D % RT_BK != 0 || D <= 0) { set_last_error("md_round_argmin_tc: D=%d must be a positive multiple of %d", D, RT_BK); return MD_ERR_ARG; }
+extern "C" __attribute__((visibility("default"))) int md_round_argmin_tc_padded(const float* x, const void* E2, const float* cst, void* x2_ws, int32_t* idx,
+                                                                              float* margin, int64_t M, int V, int D, int Dp, int mode,
+                                                                              cudaStream_t stream) {
+    if (!padded_width_ok(D, Dp)) {
+        set_last_error("md_round_argmin_tc: D=%d must be a positive multiple of 4, Dp=%d a multiple of %d >= D", D, Dp, RT_BK);
+        return MD_ERR_ARG;
+    }
     if (V <= 0 || x2_ws == nullptr || cst == nullptr || E2 == nullptr) { set_last_error("md_round_argmin_tc: bad arguments"); return MD_ERR_ARG; }
     if (mode != 0 && mode != 1) { set_last_error("md_round_argmin_tc: mode must be 0 (argmin distance) or 1 (argmax logit)"); return MD_ERR_ARG; }
     if (M == 0) return MD_OK;
     const int Vp = md_round_tc_padded_vocab(V);
     if (x != nullptr) {       // x == NULL: x2_ws already holds the split (written by the producing GEMM's epilogue)
-        split_bf16_kernel<<<ew_grid2(M * (D / 4)), 256, 0, stream>>>(x, reinterpret_cast<__nv_bfloat16*>(x2_ws), M, D, 1);
+        split_bf16_kernel<<<ew_grid2(M * (Dp / 4)), 256, 0, stream>>>(x, reinterpret_cast<__nv_bfloat16*>(x2_ws), M, D, Dp, 1);
         if (int e = check_cuda(cudaGetLastError(), "split_bf16 launch")) return e;
     }
+    // from here on the contraction runs over the padded width: the zero columns add exact zeros
     CUtensorMap tmA, tmB;
-    if (int e = make_tmap_2d(&tmA, x2_ws, 0, (uint64_t)M, 2 * D, 2 * D, RT_BM, RT_BK)) return e;
-    if (int e = make_tmap_2d(&tmB, E2, 0, (uint64_t)Vp, 2 * D, 2 * D, RT_BN, RT_BK)) return e;
+    if (int e = make_tmap_2d(&tmA, x2_ws, 0, (uint64_t)M, 2 * Dp, 2 * Dp, RT_BM, RT_BK)) return e;
+    if (int e = make_tmap_2d(&tmB, E2, 0, (uint64_t)Vp, 2 * Dp, 2 * Dp, RT_BN, RT_BK)) return e;
     RoundTcArgs a;
-    a.M = M; a.V = V; a.Vp = Vp; a.D = D; a.cst = cst; a.idx = idx; a.margin = margin;
+    a.M = M; a.V = V; a.Vp = Vp; a.D = Dp; a.cst = cst; a.idx = idx; a.margin = margin;
     static bool attr0[kMaxDevices] = {false}, attr1[kMaxDevices] = {false};
     if (ensure_dyn_smem(round_tc_kernel<0>, RT_SMEM, attr0, "cudaFuncSetAttribute(round_tc)") ||
         ensure_dyn_smem(round_tc_kernel<1>, RT_SMEM, attr1, "cudaFuncSetAttribute(round_tc)"))
@@ -285,4 +306,10 @@ extern "C" __attribute__((visibility("default"))) int md_round_argmin_tc(const f
     if (mode == 0) round_tc_kernel<0><<<grid, RT_THREADS, RT_SMEM, stream>>>(tmA, tmB, a);
     else round_tc_kernel<1><<<grid, RT_THREADS, RT_SMEM, stream>>>(tmA, tmB, a);
     return check_cuda(cudaGetLastError(), "round_tc launch");
+}
+
+extern "C" __attribute__((visibility("default"))) int md_round_argmin_tc(const float* x, const void* E2, const float* cst, void* x2_ws, int32_t* idx, float* margin,
+                                  int64_t M, int V, int D, int mode, cudaStream_t stream) {
+    if (D % RT_BK != 0 || D <= 0) { set_last_error("md_round_argmin_tc: D=%d must be a positive multiple of %d", D, RT_BK); return MD_ERR_ARG; }
+    return md_round_argmin_tc_padded(x, E2, cst, x2_ws, idx, margin, M, V, D, D, mode, stream);
 }

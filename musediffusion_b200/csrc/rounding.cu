@@ -1,14 +1,14 @@
 // Nearest-word-embedding rounding (get_efficient_knn, MuseDiffusion/models/rounding.py:21-28) and the final
 // lm_head logits + argmax (models/network.py:91-93, run/sample.py:219-220), each fused with its row reduction so the
 // [V, M] distance / [M, V] logit matrix never reaches HBM.  fp32 arithmetic (the reference's), register-blocked
-// 8 tokens x 4 vocabulary rows per thread, operands staged in padded shared memory.
+// 8 tokens x 4 vocabulary rows per thread, operands staged in padded shared memory, any D that is a multiple of 4.
 #include "common.cuh"
 #include "musediff_b200.h"
 
 namespace md {
 int num_sms();
 
-constexpr int RD = 128;          // embedding dim handled by this kernel
+constexpr int RD = 128;          // embedding columns staged per pass (wider rows are contracted in RD-column slices)
 constexpr int RT = 128;          // tokens per block
 constexpr int RV = 64;           // vocabulary rows per chunk
 constexpr int RLD = RD + 4;      // padded row stride (floats): shifts consecutive rows by 4 banks
@@ -29,12 +29,24 @@ MD_DEVINL void best_merge(Best& r, float ob, float os, int oi) {
     r.s = fminf(fminf(r.s, os), lose);
 }
 
+// rows [row0, row0 + n_rows) x columns [d0, d0 + RD) of a [rows_total, D] fp32 matrix -> smem [n_rows][RLD]; zeros outside
+MD_DEVINL void stage_slice(float* dst, const float* src, int64_t row0, int n_rows, int64_t rows_total, int D, int d0) {
+    for (int i = threadIdx.x; i < n_rows * (RD / 4); i += kRoundThreads) {
+        const int r = i >> 5, c = (i & 31) << 2;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (row0 + r < rows_total && d0 + c < D) v = *reinterpret_cast<const float4*>(src + (row0 + r) * D + d0 + c);
+        *reinterpret_cast<float4*>(dst + r * RLD + c) = v;
+    }
+}
+
 // MODE 0: key = clamp(|E_v|^2 + |x|^2 - 2 x.E_v, 0)   (argmin distance)
 // MODE 1: key = -(x.E_v + bias_v)                      (argmax logit)
+// Any D % 4 == 0: the contraction runs over RD-column slices (zero-filled past D, which adds exact zeros); every sum
+// keeps the single-slice operation order within a slice and adds the slices in order (D <= 128: one slice).
 template <int MODE>
 __global__ void __launch_bounds__(kRoundThreads, 2)
 round_kernel(const float* __restrict__ x, const float* __restrict__ E, const float* __restrict__ bias,
-             int32_t* __restrict__ out_idx, float* __restrict__ out_margin, int64_t M, int V) {
+             int32_t* __restrict__ out_idx, float* __restrict__ out_margin, int64_t M, int V, int D) {
     extern __shared__ float rsm[];
     float* xs = rsm;                    // [RT][RLD]
     float* es = xs + RT * RLD;          // [RV][RLD]
@@ -43,23 +55,23 @@ round_kernel(const float* __restrict__ x, const float* __restrict__ E, const flo
     const int tid = threadIdx.x;
     const int vg = tid & 15, tg = tid >> 4;
     const int64_t tok0 = (int64_t)blockIdx.x * RT;
+    const int n_slices = (D + RD - 1) / RD;
 
-    // ---- stage the token tile, compute |x|^2
-    for (int i = tid; i < RT * (RD / 4); i += kRoundThreads) {
-        const int r = i >> 5, c = (i & 31) << 2;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (tok0 + r < M) v = *reinterpret_cast<const float4*>(x + (tok0 + r) * RD + c);
-        *reinterpret_cast<float4*>(xs + r * RLD + c) = v;
+    // ---- |x|^2 (2 threads per token row), slice by slice; the last slice stays staged
+    float xsq = 0.f;
+    for (int sl = 0; sl < n_slices; ++sl) {
+        if (sl > 0) __syncthreads();
+        stage_slice(xs, x, tok0, RT, M, D, sl * RD);
+        __syncthreads();
+        if (MODE == 0) {
+            const int r = tid >> 1, h = tid & 1;
+            float s = 0.f;
+            for (int c = h * 64; c < h * 64 + 64; ++c) { const float v = xs[r * RLD + c]; s = fmaf(v, v, s); }
+            s += __shfl_xor_sync(0xffffffffu, s, 1);
+            xsq += s;
+        }
     }
-    __syncthreads();
-    if (MODE == 0) {
-        // 2 threads per token row
-        const int r = tid >> 1, h = tid & 1;
-        float s = 0.f;
-        for (int c = h * 64; c < h * 64 + 64; ++c) { const float v = xs[r * RLD + c]; s = fmaf(v, v, s); }
-        s += __shfl_xor_sync(0xffffffffu, s, 1);
-        if (h == 0) xn[r] = s;
-    }
+    if (MODE == 0 && (tid & 1) == 0) xn[tid >> 1] = xsq;
 
     Best best[8];
 #pragma unroll
@@ -68,48 +80,49 @@ round_kernel(const float* __restrict__ x, const float* __restrict__ E, const flo
     const int n_chunks = (V + RV - 1) / RV;
     for (int ch = 0; ch < n_chunks; ++ch) {
         const int v0 = ch * RV;
-        __syncthreads();   // previous chunk fully consumed (and xn visible on the first pass)
-        for (int i = tid; i < RV * (RD / 4); i += kRoundThreads) {
-            const int r = i >> 5, c = (i & 31) << 2;
-            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (v0 + r < V) v = *reinterpret_cast<const float4*>(E + (size_t)(v0 + r) * RD + c);
-            *reinterpret_cast<float4*>(es + r * RLD + c) = v;
-        }
-        __syncthreads();
-        {
-            // 4 threads per vocabulary row: |E_v|^2 (MODE 0) or bias (MODE 1)
-            const int r = tid >> 2, h = tid & 3;
-            float s = 0.f;
-            if (MODE == 0) {
-                for (int c = h * 32; c < h * 32 + 32; ++c) { const float v = es[r * RLD + c]; s = fmaf(v, v, s); }
-                s += __shfl_xor_sync(0xffffffffu, s, 1);
-                s += __shfl_xor_sync(0xffffffffu, s, 2);
-            } else {
-                s = (v0 + r < V) ? bias[v0 + r] : 0.f;
-            }
-            if (h == 0) en[r] = s;
-        }
         float acc[8][4];
 #pragma unroll
         for (int i = 0; i < 8; ++i)
 #pragma unroll
             for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+        float esq = 0.f;
+        for (int sl = 0; sl < n_slices; ++sl) {
+            const int d0 = sl * RD;
+            __syncthreads();   // previous slice / chunk fully consumed (and xn visible on the first pass)
+            if (n_slices > 1) stage_slice(xs, x, tok0, RT, M, D, d0);
+            stage_slice(es, E, v0, RV, V, D, d0);
+            __syncthreads();
+            if (MODE == 0) {
+                // 4 threads per vocabulary row: |E_v|^2
+                const int r = tid >> 2, h = tid & 3;
+                float s = 0.f;
+                for (int c = h * 32; c < h * 32 + 32; ++c) { const float v = es[r * RLD + c]; s = fmaf(v, v, s); }
+                s += __shfl_xor_sync(0xffffffffu, s, 1);
+                s += __shfl_xor_sync(0xffffffffu, s, 2);
+                esq += s;
+            }
+            const int dlim = min(RD, D - d0);
 #pragma unroll 4
-        for (int d = 0; d < RD; d += 4) {
-            float4 ev[4];
+            for (int d = 0; d < dlim; d += 4) {
+                float4 ev[4];
 #pragma unroll
-            for (int j = 0; j < 4; ++j) ev[j] = *reinterpret_cast<const float4*>(es + (vg + 16 * j) * RLD + d);
+                for (int j = 0; j < 4; ++j) ev[j] = *reinterpret_cast<const float4*>(es + (vg + 16 * j) * RLD + d);
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const float4 xv = *reinterpret_cast<const float4*>(xs + (tg * 8 + i) * RLD + d);
+                for (int i = 0; i < 8; ++i) {
+                    const float4 xv = *reinterpret_cast<const float4*>(xs + (tg * 8 + i) * RLD + d);
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    acc[i][j] = fmaf(xv.x, ev[j].x, acc[i][j]);
-                    acc[i][j] = fmaf(xv.y, ev[j].y, acc[i][j]);
-                    acc[i][j] = fmaf(xv.z, ev[j].z, acc[i][j]);
-                    acc[i][j] = fmaf(xv.w, ev[j].w, acc[i][j]);
+                    for (int j = 0; j < 4; ++j) {
+                        acc[i][j] = fmaf(xv.x, ev[j].x, acc[i][j]);
+                        acc[i][j] = fmaf(xv.y, ev[j].y, acc[i][j]);
+                        acc[i][j] = fmaf(xv.z, ev[j].z, acc[i][j]);
+                        acc[i][j] = fmaf(xv.w, ev[j].w, acc[i][j]);
+                    }
                 }
             }
+        }
+        {
+            const int r = tid >> 2, h = tid & 3;
+            if (h == 0) en[r] = (MODE == 0) ? esq : ((v0 + r < V) ? bias[v0 + r] : 0.f);
         }
         __syncthreads();   // en[] written above is visible
 #pragma unroll
@@ -146,13 +159,13 @@ round_kernel(const float* __restrict__ x, const float* __restrict__ E, const flo
 }
 
 template <int MODE>
-static int launch_round(const float* x, const float* E, const float* bias, int32_t* idx, float* margin, int64_t M, int V,
+static int launch_round(const float* x, const float* E, const float* bias, int32_t* idx, float* margin, int64_t M, int V, int D,
                         cudaStream_t stream) {
     auto kern = round_kernel<MODE>;
     static bool attr_set[kMaxDevices] = {false};
     if (ensure_dyn_smem(kern, kRoundSmem, attr_set, "cudaFuncSetAttribute(round)")) return MD_ERR_CUDA;
     const int64_t grid = (M + RT - 1) / RT;
-    kern<<<(unsigned)grid, kRoundThreads, kRoundSmem, stream>>>(x, E, bias, idx, margin, M, V);
+    kern<<<(unsigned)grid, kRoundThreads, kRoundSmem, stream>>>(x, E, bias, idx, margin, M, V, D);
     return check_cuda(cudaGetLastError(), "round launch");
 }
 
@@ -162,16 +175,16 @@ using namespace md;
 
 extern "C" __attribute__((visibility("default"))) int md_round_argmin(const float* x, const float* E, int32_t* idx, float* margin, int64_t M, int V, int D,
                                cudaStream_t stream) {
-    if (D != RD) { set_last_error("md_round_argmin: D=%d unsupported (kernel is specialised for D=%d)", D, RD); return MD_ERR_ARG; }
+    if (D <= 0 || D % 4 != 0) { set_last_error("md_round_argmin: D=%d must be a positive multiple of 4", D); return MD_ERR_ARG; }
     if (V <= 0) { set_last_error("md_round_argmin: empty vocabulary"); return MD_ERR_ARG; }
     if (M == 0) return MD_OK;
-    return launch_round<0>(x, E, nullptr, idx, margin, M, V, stream);
+    return launch_round<0>(x, E, nullptr, idx, margin, M, V, D, stream);
 }
 
 extern "C" __attribute__((visibility("default"))) int md_logits_argmax(const float* x, const float* E, const float* bias, int32_t* tok, float* margin, int64_t M,
                                 int V, int D, cudaStream_t stream) {
-    if (D != RD) { set_last_error("md_logits_argmax: D=%d unsupported (kernel is specialised for D=%d)", D, RD); return MD_ERR_ARG; }
+    if (D <= 0 || D % 4 != 0) { set_last_error("md_logits_argmax: D=%d must be a positive multiple of 4", D); return MD_ERR_ARG; }
     if (V <= 0 || bias == nullptr) { set_last_error("md_logits_argmax: bad arguments"); return MD_ERR_ARG; }
     if (M == 0) return MD_OK;
-    return launch_round<1>(x, E, bias, tok, margin, M, V, stream);
+    return launch_round<1>(x, E, bias, tok, margin, M, V, D, stream);
 }

@@ -59,6 +59,11 @@ def _cast_f32_bf16(x, out):
     launch("md_cast_f32_bf16", _p(x), _p(out), x.numel(), _stream())
 
 
+def _cast_f32_bf16_ld(x, out):
+    D = x.shape[-1]
+    launch("md_cast_f32_bf16_ld", _p(x), _p(out), x.numel() // D, D, out.shape[-1], _stream())
+
+
 def _cast_bf16_f32(x, out):
     launch("md_cast_bf16_f32", _p(x), _p(out), x.numel(), _stream())
 
@@ -88,6 +93,13 @@ def _linear_bf16(A, W, bias, out, epilogue, pos, temb, temb_stride, L):
     N = W.shape[0]                                     # (the split epilogue writes out = bf16 [M, 2N])
     launch("md_linear_bf16", _p(A), _p(W), _p(bias), _p(out), M, N, K, epilogue, int(out.dtype == torch.float32), _p(pos), _p(temb),
            temb_stride, L, _stream(), detail="%dx%dx%d epi=%d" % (M, N, K, epilogue))
+
+
+def _linear_bf16_cols(A, W, bias, out, epilogue, pos, temb, temb_stride, L):
+    M, K = A.shape
+    N = W.shape[0]
+    launch("md_linear_bf16_cols", _p(A), _p(W), _p(bias), _p(out), M, N, K, out.shape[-1], epilogue, int(out.dtype == torch.float32),
+           _p(pos), _p(temb), temb_stride, L, _stream(), detail="%dx%dx%d epi=%d cols=%d" % (M, N, K, epilogue, out.shape[-1]))
 
 
 def _attention_bf16(qkv, out, B, L, NH):
@@ -121,6 +133,15 @@ def _round_argmin_tc(x, E2, cst, ws, idx, margin, V, mode):
     launch("md_round_argmin_tc", _p(x), _p(E2), _p(cst), _p(ws), _p(idx), _p(margin), idx.numel(), V, D, mode, _stream())
 
 
+def _embed_split_padded(E, E2, sqnorm, E_clamped):
+    launch("md_embed_split_padded", _p(E), E.shape[0], E.shape[1], E2.shape[1] // 2, _p(E2), _p(sqnorm), _p(E_clamped), _stream())
+
+
+def _round_argmin_tc_padded(x, E2, cst, ws, idx, margin, V, D, mode):
+    launch("md_round_argmin_tc_padded", _p(x), _p(E2), _p(cst), _p(ws), _p(idx), _p(margin), idx.numel(), V, D, E2.shape[1] // 2, mode,
+           _stream())
+
+
 # ------------------------------------------------------------------------------------------------ diffusion steps
 def _posterior_step(x_t, idx, pred, E, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask_tok_stride, mask_d_stride,
                     x_start, out, out_bf16, pred_out, mean_out, mode, eta, clip, top_p, step_counter_dev):
@@ -128,6 +149,15 @@ def _posterior_step(x_t, idx, pred, E, noise, seed, step_counter, seq_offset, t,
     launch("md_posterior_step", _p(x_t), _p(idx), _p(pred), _p(E), _p(noise), seed & _U64, step_counter & _U64, seq_offset, _p(t),
            t_stride, _p(mask), mask_tok_stride, mask_d_stride, _p(x_start), _p(out), _p(out_bf16), _p(pred_out), _p(mean_out),
            B, L, D, mode, float(eta), int(clip), float(top_p), _p(step_counter_dev), _stream())
+
+
+def _posterior_step_ld(x_t, idx, pred, E, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask_tok_stride, mask_d_stride,
+                       x_start, out, out_bf16, pred_out, mean_out, mode, eta, clip, top_p, step_counter_dev):
+    B, L, D = x_t.shape
+    launch("md_posterior_step_ld", _p(x_t), _p(idx), _p(pred), _p(E), _p(noise), seed & _U64, step_counter & _U64, seq_offset, _p(t),
+           t_stride, _p(mask), mask_tok_stride, mask_d_stride, _p(x_start), _p(out), _p(out_bf16),
+           out_bf16.shape[-1] if out_bf16 is not None else D, _p(pred_out), _p(mean_out), B, L, D, mode, float(eta), int(clip),
+           float(top_p), _p(step_counter_dev), _stream())
 
 
 def _xstart_from_eps(x_t, eps, t, t_stride, out):
@@ -139,6 +169,12 @@ def _q_sample(x0, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask
     B, L, D = x0.shape
     launch("md_q_sample", _p(x0), _p(noise), seed & _U64, step_counter & _U64, seq_offset, _p(t), t_stride, _p(mask), mask_tok_stride,
            mask_d_stride, _p(out), _p(out_bf16), B, L, D, _stream())
+
+
+def _q_sample_ld(x0, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask_tok_stride, mask_d_stride, out, out_bf16):
+    B, L, D = x0.shape
+    launch("md_q_sample_ld", _p(x0), _p(noise), seed & _U64, step_counter & _U64, seq_offset, _p(t), t_stride, _p(mask), mask_tok_stride,
+           mask_d_stride, _p(out), _p(out_bf16), out_bf16.shape[-1] if out_bf16 is not None else D, B, L, D, _stream())
 
 
 def _fill_normal(out, seed, step_counter, elem_offset, top_p):
@@ -173,6 +209,7 @@ def _onnc(vectors, msim, most_sim):
 
 
 _define("cast_f32_bf16(Tensor x, Tensor(a!) out) -> ()", _cast_f32_bf16)
+_define("cast_f32_bf16_ld(Tensor x, Tensor(a!) out) -> ()", _cast_f32_bf16_ld)
 _define("cast_bf16_f32(Tensor x, Tensor(a!) out) -> ()", _cast_bf16_f32)
 _define("add_pos_time(Tensor x, Tensor pos, Tensor temb, int temb_stride, int L, Tensor(a!) out) -> ()", _add_pos_time)
 _define("embed_gather(Tensor E, Tensor ids, Tensor(a!) out) -> ()", _embed_gather)
@@ -180,6 +217,8 @@ _define("timestep_mlp(Tensor t, Tensor W0, Tensor b0, Tensor W2, Tensor b2, Tens
 _define("layernorm_bf16(Tensor x, Tensor? resid, Tensor gamma, Tensor beta, float eps, Tensor(a!) out) -> ()", _layernorm_bf16)
 _define("linear_bf16(Tensor A, Tensor W, Tensor? bias, Tensor(a!) out, int epilogue, Tensor? pos, Tensor? temb, int temb_stride, "
         "int L) -> ()", _linear_bf16)
+_define("linear_bf16_cols(Tensor A, Tensor W, Tensor? bias, Tensor(a!) out, int epilogue, Tensor? pos, Tensor? temb, "
+        "int temb_stride, int L) -> ()", _linear_bf16_cols)
 _define("attention_bf16(Tensor qkv, Tensor(a!) out, int B, int L, int NH) -> ()", _attention_bf16)
 _define("round_argmin(Tensor x, Tensor E, Tensor(a!) idx, Tensor(b!)? margin) -> ()", _round_argmin)
 _define("logits_argmax(Tensor x, Tensor E, Tensor bias, Tensor(a!) tok, Tensor(b!)? margin) -> ()", _logits_argmax)
@@ -188,13 +227,22 @@ _define("embed_split(Tensor E, Tensor(a!) E2, Tensor(b!) sqnorm, Tensor(c!)? E_c
 _define("dist_scores(Tensor x, Tensor dot, Tensor esq, Tensor(a!) out) -> ()", _dist_scores)
 _define("round_argmin_tc(Tensor? x, Tensor E2, Tensor cst, Tensor(a!) ws, Tensor(b!) idx, Tensor(c!)? margin, int V, int mode) -> ()",
         _round_argmin_tc)
+_define("embed_split_padded(Tensor E, Tensor(a!) E2, Tensor(b!) sqnorm, Tensor(c!)? E_clamped) -> ()", _embed_split_padded)
+_define("round_argmin_tc_padded(Tensor? x, Tensor E2, Tensor cst, Tensor(a!) ws, Tensor(b!) idx, Tensor(c!)? margin, int V, int D, "
+        "int mode) -> ()", _round_argmin_tc_padded)
 _define("posterior_step(Tensor x_t, Tensor? idx, Tensor? pred, Tensor? E, Tensor? noise, int seed, int step_counter, int seq_offset, "
         "Tensor t, int t_stride, Tensor? mask, int mask_tok_stride, int mask_d_stride, Tensor? x_start, Tensor(a!) out, "
         "Tensor(b!)? out_bf16, Tensor(c!)? pred_out, Tensor(d!)? mean_out, int mode, float eta, int clip, float top_p, "
         "Tensor? step_counter_dev) -> ()", _posterior_step)
+_define("posterior_step_ld(Tensor x_t, Tensor? idx, Tensor? pred, Tensor? E, Tensor? noise, int seed, int step_counter, "
+        "int seq_offset, Tensor t, int t_stride, Tensor? mask, int mask_tok_stride, int mask_d_stride, Tensor? x_start, Tensor(a!) out, "
+        "Tensor(b!)? out_bf16, Tensor(c!)? pred_out, Tensor(d!)? mean_out, int mode, float eta, int clip, float top_p, "
+        "Tensor? step_counter_dev) -> ()", _posterior_step_ld)
 _define("xstart_from_eps(Tensor x_t, Tensor eps, Tensor t, int t_stride, Tensor(a!) out) -> ()", _xstart_from_eps)
 _define("q_sample(Tensor x0, Tensor? noise, int seed, int step_counter, int seq_offset, Tensor? t, int t_stride, Tensor? mask, "
         "int mask_tok_stride, int mask_d_stride, Tensor(a!) out, Tensor(b!)? out_bf16) -> ()", _q_sample)
+_define("q_sample_ld(Tensor x0, Tensor? noise, int seed, int step_counter, int seq_offset, Tensor? t, int t_stride, Tensor? mask, "
+        "int mask_tok_stride, int mask_d_stride, Tensor(a!) out, Tensor(b!)? out_bf16) -> ()", _q_sample_ld)
 _define("fill_normal(Tensor(a!) out, int seed, int step_counter, int elem_offset, float top_p) -> ()", _fill_normal)
 _define("step_advance(Tensor(a!) cursor, Tensor t_idx, Tensor t_model, Tensor(b!) t_cur, Tensor(c!) tm_cur, Tensor(d!) ctr_cur, "
         "int ctr_base) -> ()", _step_advance)
@@ -206,7 +254,9 @@ _define("sequence_metrics(Tensor notes, Tensor note_len, Tensor meta, Tensor(a!)
         _sequence_metrics)
 _define("onnc(Tensor vectors, Tensor(a!)? msim, Tensor(b!) most_sim) -> ()", _onnc)
 
-OP_NAMES = ["cast_f32_bf16", "cast_bf16_f32", "add_pos_time", "embed_gather", "timestep_mlp", "layernorm_bf16", "linear_bf16", "attention_bf16", "round_argmin",
-            "logits_argmax", "split_bf16", "dist_scores", "embed_split", "round_argmin_tc", "posterior_step", "xstart_from_eps", "q_sample",
-            "fill_normal", "step_advance", "decode_prepare", "merge_and_mask", "sequence_metrics", "onnc"]
+OP_NAMES = ["cast_f32_bf16", "cast_f32_bf16_ld", "cast_bf16_f32", "add_pos_time", "embed_gather", "timestep_mlp", "layernorm_bf16",
+            "linear_bf16", "linear_bf16_cols", "attention_bf16", "round_argmin", "logits_argmax", "split_bf16", "dist_scores",
+            "embed_split", "embed_split_padded", "round_argmin_tc", "round_argmin_tc_padded", "posterior_step", "posterior_step_ld",
+            "xstart_from_eps", "q_sample", "q_sample_ld", "fill_normal", "step_advance", "decode_prepare", "merge_and_mask",
+            "sequence_metrics", "onnc"]
 ops = getattr(torch.ops, NAMESPACE)

@@ -396,7 +396,9 @@ class GaussianDiffusion:
             if fast is not None:
                 t_arg = t_idx[k:k + 1]
                 model_output = fast.denoise(x, t_model[k:k + 1], x_bf16=x_bf16, uniform_t=True)
-                x_bf16 = torch.empty_like(x, dtype=torch.bfloat16)
+                Dp = fast.weight_pack().Dp          # padded operand width: its pad columns stay zero, the kernel never writes them
+                x_bf16 = (torch.empty_like(x, dtype=torch.bfloat16) if Dp == x.shape[-1]
+                          else torch.zeros(x.shape[:-1] + (Dp,), dtype=torch.bfloat16, device=x.device))
             else:
                 t_arg, model_output = t_idx[k:k + 1].long().expand(B), None
             x, pred, mean = self._step(mode, model, x, t_arg, clip_denoised, fn, model_kwargs, top_p, mask, x_start, eta,
@@ -407,19 +409,20 @@ class GaussianDiffusion:
         """The chain as one fixed reverse-step body whose per-step inputs live in device memory: `md_step_advance` moves a
         cursor over the index tables and publishes the schedule index, the denoiser's timestep value and the Philox
         counter of the step, which the posterior kernel reads.  x_t is updated in place (the posterior kernel is
-        elementwise) and its bf16 copy feeds the next step's first GEMM.
+        elementwise) and its bf16 copy, padded to the operand width Dp with zero columns, feeds the next step's first GEMM.
         `capture`: the first step runs eagerly (one-time set-up: shared-memory attributes, weight pack, tensor maps), the
         second is captured as a CUDA graph (SURVEY.md section 7 step 7) and every later step replays it.  Otherwise every
         step launches the same body directly, so per-launch timings measure the kernels a replay runs."""
         dev = x.device
         self._upload_schedule()
         x = x.clone()                                   # updated in place: never the caller's tensor
-        xb = ops.cast_bf16(x)
+        pk = fast.weight_pack()
+        xb = ops.cast_bf16(x, width=pk.Dp)
         # x0-predicting model: the last Linear emits the [hi | lo] bf16 split that the rounding contraction consumes, the fp32
         # model output never exists; an eps-predicting model needs it in fp32 for x0 = sr x_t - srm1 eps first
-        use_split = self.predict_xstart and fast.weight_pack().has_down
+        use_split = self.predict_xstart and pk.has_down
         mo = torch.empty_like(x) if not use_split else None
-        mo_split = torch.empty(x.shape[:-1] + (2 * x.shape[-1],), dtype=torch.bfloat16, device=dev) if use_split else None
+        mo_split = torch.empty(x.shape[:-1] + (2 * pk.Dp,), dtype=torch.bfloat16, device=dev) if use_split else None
         cursor = torch.zeros(1, dtype=torch.int32, device=dev)
         t_cur = torch.zeros(1, dtype=torch.int32, device=dev)
         tm_cur = torch.zeros(1, dtype=torch.float32, device=dev)

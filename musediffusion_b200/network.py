@@ -66,9 +66,22 @@ class _Encoder(nn.Module):
                                     for _ in range(cfg.num_hidden_layers)])
 
 
+def _zero_pad(t, rows, cols):
+    """t [r, c] (or [r]) zero-extended to [rows, cols] (or [rows])."""
+    if t.shape[0] == rows and (t.dim() == 1 or t.shape[1] == cols):
+        return t
+    out = torch.zeros((rows,) if t.dim() == 1 else (rows, cols), dtype=t.dtype, device=t.device)
+    out[tuple(slice(0, n) for n in t.shape)] = t
+    return out
+
+
 class WeightPack:
     """Device-resident bf16 / fp32 weights in the layout the kernels consume: built from the parameters once per parameter
-    version (`checkpoint.pack_tensors`), or served straight from a packed weight file (`checkpoint.load_pack`)."""
+    version (`checkpoint.pack_tensors`), or served straight from a packed weight file (`checkpoint.load_pack`).
+
+    A width D that is not a multiple of 64 is zero-padded to Dp = ops.padded_width(D) here, at load time: up1_w
+    [H, Dp] (zero columns: the pad columns of the input contribute nothing), dn2_w [Dp, H] and dn2_b [Dp] (zero rows: the
+    pad columns of the output, and so of its [hi | lo] split, are exactly 0).  The embedding E stays [V, D]."""
 
     def __init__(self, model, tensors=None):
         dev = model.word_embedding.weight.device if tensors is None else tensors["E"].device
@@ -89,6 +102,12 @@ class WeightPack:
         self.has_up, self.has_down = self.up1_w is not None, self.dn1_w is not None
         if self.has_up != (model.input_dims != model.hidden_size) or self.has_down != (model.output_dims != model.hidden_size):
             raise ValueError("weight pack and model disagree about input_up_proj / output_down_proj")
+        self.D = self.E.shape[1]
+        self.Dp = ops.padded_width(self.D) if self.has_up else self.D         # no projections: D == H, a multiple of 64
+        if self.has_up:
+            self.up1_w = _zero_pad(self.up1_w, self.H, self.Dp)
+        if self.has_down:
+            self.dn2_w, self.dn2_b = _zero_pad(self.dn2_w, self.Dp, self.H), _zero_pad(self.dn2_b, self.Dp, 0)
         self.layers = []
         i = 0
         while "l%d.wqkv" % i in tensors:
@@ -116,10 +135,10 @@ class WeightPack:
 class Workspace:
     """Activation buffers for one token count M (reused across steps: nothing is allocated inside the loop)."""
 
-    def __init__(self, M, D, H, F, dev):
+    def __init__(self, M, Dp, H, F, dev):
         bf = lambda *s: torch.empty(s, dtype=torch.bfloat16, device=dev)
         self.M = M
-        self.xb = bf(M, D)
+        self.xb = bf(M, Dp)
         self.a = bf(M, H)
         self.b = bf(M, H)
         self.c = bf(M, H)
@@ -135,6 +154,10 @@ class TransformerNetModel(nn.Module):
     def __init__(self, input_dims, output_dims, hidden_t_dim, vocab_size, seq_len, dropout=0.1, logits_mode=1,
                  encoder_config=None):
         super().__init__()
+        for name, d in (("input_dims", input_dims), ("output_dims", output_dims)):
+            if int(d) <= 0 or int(d) % 4:
+                raise ValueError("%s (hidden_dim) = %d is not supported: the embedding width must be a positive multiple of 4 "
+                                 "(the kernels move rows in float4 groups)" % (name, d))
         cfg = SimpleNamespace(**{**BERT_BASE, **(encoder_config or {})})
         cfg.max_position_embeddings = seq_len
         cfg.vocab_size = vocab_size
@@ -217,7 +240,7 @@ class TransformerNetModel(nn.Module):
         ws = self._ws.get(M)
         if ws is None:
             pk = self.weight_pack()
-            self._ws = {M: Workspace(M, self.input_dims, pk.H, self.config.intermediate_size, pk.device)}
+            self._ws = {M: Workspace(M, pk.Dp, pk.H, self.config.intermediate_size, pk.device)}
             ws = self._ws[M]
         return ws
 
@@ -283,10 +306,10 @@ class TransformerNetModel(nn.Module):
         return -(-B // n_pass)
 
     def denoise(self, x, timesteps, x_bf16=None, uniform_t=False, out=None, split_out=None):
-        """The CUDA forward.  `x_bf16`: optional bf16 copy of x already produced by the posterior-step kernel;
-        `uniform_t`: all rows share timesteps[0] (true inside the sampling loops) -> one time-embedding row;
-        `split_out`: bf16 [B, L, 2D] — the last Linear then writes the [hi | lo] split of the output (operand of the
-        tensor-core rounding) INSTEAD of the fp32 tensor, and `split_out` is returned."""
+        """The CUDA forward.  `x_bf16`: optional bf16 copy of x already produced by the posterior-step kernel, [B, L, Dp]
+        (Dp = ops.padded_width(D), zero columns D..Dp-1); `uniform_t`: all rows share timesteps[0] (true inside the sampling
+        loops) -> one time-embedding row; `split_out`: bf16 [B, L, 2Dp] — the last Linear then writes the [hi | 0 | lo | 0]
+        split of the output (operand of the tensor-core rounding) INSTEAD of the fp32 tensor, and `split_out` is returned."""
         pk = self.weight_pack()
         if not x.is_cuda:
             raise _lib.MuseDiffLibraryError("TransformerNetModel.forward needs CUDA tensors (no CPU path)")
@@ -301,14 +324,16 @@ class TransformerNetModel(nn.Module):
                 raise ValueError("timesteps has %d entries for a batch of %d sequences" % (t.numel(), B))
         if split_out is not None and not pk.has_down:
             raise ValueError("split_out needs the output_down_proj GEMM (hidden_dim != hidden size)")
+        Dp = pk.Dp
         if split_out is not None:
-            out = split_out.view(B, L, 2 * D)
+            out = split_out.view(B, L, 2 * Dp)
         else:
             if out is None:
                 out = torch.empty((B, L, D), dtype=torch.float32, device=x.device)
             out = out.view(B, L, D)
         if pk.has_up:
-            xb = x_bf16.view(B, L, D) if x_bf16 is not None else ops.cast_bf16(x.reshape(B * L, D).float()).view(B, L, D)
+            xb = (x_bf16.view(B, L, Dp) if x_bf16 is not None
+                  else ops.cast_bf16(x.reshape(B * L, D).float(), width=Dp).view(B, L, Dp))
         else:
             xb = x.float().contiguous()                   # emb_x = x (network.py:143-144): the fp32 state feeds the pre-LN sum
         temb = ops.timestep_mlp(t[:1] if uniform_t else t, pk.t0_w, pk.t0_b, pk.t2_w, pk.t2_b)
@@ -320,18 +345,18 @@ class TransformerNetModel(nn.Module):
         return out
 
     def _encoder_pass(self, pk, ws, xb, temb, uniform_t, out, split=False):
-        """network.py:141-157 for a contiguous slice of sequences: xb bf16 [b, L, D] -> out fp32 [b, L, D]
-        (split: bf16 [b, L, 2D] = [hi | lo])."""
-        b, L, D = xb.shape
+        """network.py:141-157 for a contiguous slice of sequences: xb bf16 [b, L, Dp] -> out fp32 [b, L, D]
+        (split: bf16 [b, L, 2Dp] = [hi | 0 | lo | 0])."""
+        b, L, Dp = xb.shape
         M, H = b * L, pk.H
         E = _lib
         a, bb, c, qkv, mid = ws.a[:M], ws.b[:M], ws.c[:M], ws.qkv[:M], ws.mid[:M]
         if pk.has_up:
-            ops.linear(xb.view(M, D), pk.up1_w, pk.up1_b, E.EPI_BIAS_TANH, out=a)
+            ops.linear(xb.view(M, Dp), pk.up1_w, pk.up1_b, E.EPI_BIAS_TANH, out=a)
             ops.linear(a, pk.up2_w, pk.up2_b, E.EPI_BIAS_POS_TIME, pos=pk.pos, temb=temb,
                        temb_stride=0 if uniform_t else H, L=L, out=bb)
         else:
-            ops.add_pos_time(xb.view(M, D), pk.pos, temb, 0 if uniform_t else H, L, bb)
+            ops.add_pos_time(xb.view(M, Dp), pk.pos, temb, 0 if uniform_t else H, L, bb)
         h, h1, pre = a, c, bb
         ops.layernorm(pre, pk.ln_g, pk.ln_b, pk.eps, out=h)
         for ly in pk.layers:
@@ -343,10 +368,10 @@ class TransformerNetModel(nn.Module):
             ops.linear(mid, ly.w2, ly.b2, E.EPI_BIAS, out=pre)
             ops.layernorm(pre, ly.g2, ly.b2n, pk.eps, resid=h1, out=h)       # LN(dense(mid) + h1)
         if not pk.has_down:
-            ops.cast_f32(h, out=out.view(M, D))           # h.type(x.dtype) of the last hidden state (network.py:155-157)
+            ops.cast_f32(h, out=out.view(M, -1))          # h.type(x.dtype) of the last hidden state (network.py:155-157)
             return
         ops.linear(h, pk.dn1_w, pk.dn1_b, E.EPI_BIAS_TANH, out=h1)
         if split:
-            ops.linear(h1, pk.dn2_w, pk.dn2_b, E.EPI_BIAS_SPLIT, out=out.view(M, 2 * D))
-        else:
-            ops.linear(h1, pk.dn2_w, pk.dn2_b, E.EPI_BIAS, out=out.view(M, D))
+            ops.linear(h1, pk.dn2_w, pk.dn2_b, E.EPI_BIAS_SPLIT, out=out.view(M, 2 * Dp))
+        else:                                             # N = Dp, the D real columns are stored
+            ops.linear(h1, pk.dn2_w, pk.dn2_b, E.EPI_BIAS, out=out.view(M, -1))

@@ -75,12 +75,25 @@ def set_schedule(tables64, key=None):
     _current_schedule_key[torch.cuda.current_device()] = key
 
 
+def padded_width(D):
+    """Dp: the width of the bf16 tensor-core operands that stand for a D-wide state or embedding (the first Linear's A
+    operand, the [hi | lo] rounding operands, W_up1's columns, W_dn2's rows).  D rounded up to a multiple of 64; the
+    columns D..Dp-1 hold zeros, which leaves every contraction unchanged."""
+    return -(-int(D) // 64) * 64
+
+
 # ------------------------------------------------------------------------------------------------ elementwise
-def cast_bf16(x):
+def cast_bf16(x, width=None):
+    """fp32 [..., D] -> bf16 [..., width] (width defaults to D; columns D..width-1 are zero)."""
     x = _c(x, torch.float32)
-    out = torch.empty(x.shape, dtype=BF16, device=x.device)
+    D = x.shape[-1]
     _cu(x)
-    K.cast_f32_bf16(x, out)
+    if width is None or width == D:
+        out = torch.empty(x.shape, dtype=BF16, device=x.device)
+        K.cast_f32_bf16(x, out)
+    else:
+        out = torch.zeros(x.shape[:-1] + (width,), dtype=BF16, device=x.device)
+        K.cast_f32_bf16_ld(x, out)
     return out
 
 
@@ -138,7 +151,8 @@ def layernorm(x, gamma, beta, eps, resid=None, out=None):
 
 # ------------------------------------------------------------------------------------------------ contractions
 def linear(A, W, bias, epilogue=_lib.EPI_BIAS, out_dtype=BF16, pos=None, temb=None, temb_stride=0, L=0, out=None):
-    """out[M,N] = epi(A[M,K] @ W[N,K]^T + bias)."""
+    """out[M,N] = epi(A[M,K] @ W[N,K]^T + bias).  An `out` narrower than N receives the first out.shape[-1] columns
+    (md_linear_bf16_cols: how a model whose width is padded to Dp writes its D real output columns)."""
     assert A.dtype == BF16 and W.dtype == BF16 and A.is_contiguous() and W.is_contiguous()
     M, Kd = A.shape
     N = W.shape[0]
@@ -148,7 +162,10 @@ def linear(A, W, bias, epilogue=_lib.EPI_BIAS, out_dtype=BF16, pos=None, temb=No
     if epilogue == _lib.EPI_BIAS_SPLIT and (out.dtype != BF16 or out.shape[-1] != 2 * N):
         raise _lib.MuseDiffLibraryError("md_linear_bf16: the split epilogue writes bf16 [M, 2N]")
     _cu(A, W, bias, out, pos, temb)
-    K.linear_bf16(A, W, bias, out, epilogue, pos, temb, temb_stride, L)
+    if epilogue != _lib.EPI_BIAS_SPLIT and out.shape[-1] != N:
+        K.linear_bf16_cols(A, W, bias, out, epilogue, pos, temb, temb_stride, L)
+    else:
+        K.linear_bf16(A, W, bias, out, epilogue, pos, temb, temb_stride, L)
     return out
 
 
@@ -212,18 +229,23 @@ def dist_scores(x, dot, esq, V):
 
 
 class SplitEmbedding:
-    """bf16 [Vp, 2D] = [Eh | El] split of an embedding matrix + |E_v|^2, built once per matrix version
-    (md_embed_split); `logit_cst(bias)` gives the padded per-column constants of the argmax-logits mode."""
+    """bf16 [Vp, 2Dp] = [Eh | 0 | El | 0] split of an embedding matrix (Dp = padded_width(D)) + |E_v|^2, built once per
+    matrix version (md_embed_split, md_embed_split_padded when D is not a multiple of 64); `logit_cst(bias)` gives the
+    padded per-column constants of the argmax-logits mode."""
 
     def __init__(self, E):
         E = _c(E.detach(), torch.float32)
         self.V, self.D = E.shape
+        self.Dp = padded_width(self.D)
         self.Vp = _lib.lib.md_round_tc_padded_vocab(self.V)
-        self.E2 = torch.empty((self.Vp, 2 * self.D), dtype=BF16, device=E.device)
+        self.E2 = torch.empty((self.Vp, 2 * self.Dp), dtype=BF16, device=E.device)
         self.sqnorm = torch.empty((self.Vp,), dtype=torch.float32, device=E.device)
         self.E_clamped = torch.empty_like(E)      # clamp(E, -1, 1): what clip_denoised makes of a rounded x0 (diffusion.py:323-324)
         _cu(E)
-        K.embed_split(E, self.E2, self.sqnorm, self.E_clamped)
+        if self.Dp == self.D:
+            K.embed_split(E, self.E2, self.sqnorm, self.E_clamped)
+        else:
+            K.embed_split_padded(E, self.E2, self.sqnorm, self.E_clamped)
         self._ws = {}
 
     def logit_cst(self, bias):
@@ -234,7 +256,7 @@ class SplitEmbedding:
     def workspace(self, M):
         ws = self._ws.get(M)
         if ws is None:
-            self._ws = {M: torch.empty((M, 2 * self.D), dtype=BF16, device=self.E2.device)}
+            self._ws = {M: torch.empty((M, 2 * self.Dp), dtype=BF16, device=self.E2.device)}
             ws = self._ws[M]
         return ws
 
@@ -258,11 +280,12 @@ def split_embedding(E):
 
 def round_argmin_tc(x, se, cst=None, mode=0, want_margin=False, out=None, presplit=None):
     """tensor-core nearest-embedding ids (mode 0, cst = |E|^2) or argmax-logit ids (mode 1, cst = padded bias).
-    `presplit`: bf16 [M, 2D] = [hi | lo] of x already written by the producing GEMM (EPI_BIAS_SPLIT); x is then ignored."""
+    x: fp32 [..., D].  `presplit`: bf16 [M, 2Dp] = [hi | 0 | lo | 0] of x already written by the producing GEMM
+    (EPI_BIAS_SPLIT with N = Dp); x is then ignored."""
     if presplit is not None:
-        assert presplit.dtype == BF16 and presplit.is_contiguous() and presplit.shape[-1] == 2 * se.D
-        M = presplit.numel() // (2 * se.D)
-        x, ws, dev = None, presplit.view(M, 2 * se.D), presplit.device
+        assert presplit.dtype == BF16 and presplit.is_contiguous() and presplit.shape[-1] == 2 * se.Dp
+        M = presplit.numel() // (2 * se.Dp)
+        x, ws, dev = None, presplit.view(M, 2 * se.Dp), presplit.device
     else:
         x = _c(x, torch.float32)
         M = x.numel() // se.D
@@ -270,7 +293,11 @@ def round_argmin_tc(x, se, cst=None, mode=0, want_margin=False, out=None, prespl
     idx = out if out is not None else torch.empty((M,), dtype=torch.int32, device=dev)
     margin = torch.empty((M,), dtype=torch.float32, device=dev) if want_margin else None
     _cu(x, ws)
-    K.round_argmin_tc(x, se.E2, se.sqnorm if cst is None else cst, ws, idx, margin, se.V, mode)
+    cst = se.sqnorm if cst is None else cst
+    if se.Dp == se.D:
+        K.round_argmin_tc(x, se.E2, cst, ws, idx, margin, se.V, mode)
+    else:
+        K.round_argmin_tc_padded(x, se.E2, cst, ws, idx, margin, se.V, se.D, mode)
     return (idx, margin) if want_margin else idx
 
 
@@ -304,7 +331,8 @@ def _t_args(t, B):
 def posterior_step(x_t, t, mode, idx=None, pred=None, E=None, noise=None, seed=0, step_counter=0, seq_offset=0,
                    mask=None, x_start=None, eta=0.0, clip=True, top_p=0.0, out=None, out_bf16=None, pred_out=None,
                    mean_out=None, step_counter_dev=None):
-    """clip: False / True as diffusion.py:323-324, or 2 = `E` already holds clamp(E, -1, 1) (SplitEmbedding.E_clamped)."""
+    """clip: False / True as diffusion.py:323-324, or 2 = `E` already holds clamp(E, -1, 1) (SplitEmbedding.E_clamped).
+    out_bf16: bf16 [B, L, D], or [B, L, Dp] with zeroed columns D..Dp-1 (the padded first-GEMM operand)."""
     x_t = _c(x_t, torch.float32)
     B, L, D = x_t.shape
     t, t_stride = _t_args(t, B)
@@ -322,7 +350,8 @@ def posterior_step(x_t, t, mode, idx=None, pred=None, E=None, noise=None, seed=0
     if (idx is None) == (pred is None):
         raise _lib.MuseDiffLibraryError("md_posterior_step: exactly one of idx / pred_in")
     _cu(x_t, idx, pred, E, noise, t, mask_t, x_start, out, out_bf16, pred_out, mean_out, step_counter_dev)
-    K.posterior_step(x_t, idx, pred, E, noise, _s64(seed), _s64(step_counter), int(seq_offset), t, t_stride, mask_t, ts, ds, x_start,
+    step = K.posterior_step if out_bf16 is None or out_bf16.shape[-1] == D else K.posterior_step_ld
+    step(x_t, idx, pred, E, noise, _s64(seed), _s64(step_counter), int(seq_offset), t, t_stride, mask_t, ts, ds, x_start,
                      out, out_bf16, pred_out, mean_out, mode, float(eta), int(clip), float(top_p or 0.0), step_counter_dev)
     return out
 
@@ -339,7 +368,7 @@ def xstart_from_eps(x_t, eps, t):
 
 
 def q_sample(x0, t=None, noise=None, seed=0, step_counter=0, seq_offset=0, mask=None, out_bf16=None):
-    """t=None -> pure-noise initialisation (generation mode)."""
+    """t=None -> pure-noise initialisation (generation mode).  out_bf16 as in posterior_step."""
     x0 = _c(x0, torch.float32)
     B, L, D = x0.shape
     keep, mask_t, ts, ds = _mask_args(mask, B, L, D)
@@ -348,7 +377,8 @@ def q_sample(x0, t=None, noise=None, seed=0, step_counter=0, seq_offset=0, mask=
         noise = _c(noise, torch.float32)
     tt, t_stride = _t_args(t, B) if t is not None else (None, 0)
     _cu(x0, noise, tt, mask_t, out_bf16)
-    K.q_sample(x0, noise, _s64(seed), _s64(step_counter), int(seq_offset), tt, t_stride, mask_t, ts, ds, out, out_bf16)
+    qs = K.q_sample if out_bf16 is None or out_bf16.shape[-1] == D else K.q_sample_ld
+    qs(x0, noise, _s64(seed), _s64(step_counter), int(seq_offset), tt, t_stride, mask_t, ts, ds, out, out_bf16)
     return out
 
 
