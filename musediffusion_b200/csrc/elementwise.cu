@@ -633,7 +633,9 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
         for (int j = 0; j < VEC * 8; ++j) s += v[j];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        const float mean = s * (1.0f / H);
+        // correctly rounded: for a constant row c the sum H c is exact, and s / H is then exactly c at every width
+        // (s * fl(1/H) is not for H = 1792, where a constant row came out as beta +- gamma * O(1) instead of beta)
+        const float mean = __fdiv_rn(s, (float)H);
         float q = 0.f;
 #pragma unroll
         for (int j = 0; j < VEC * 8; ++j) { const float dlt = v[j] - mean; q = fmaf(dlt, dlt, q); }
