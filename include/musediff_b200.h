@@ -98,7 +98,10 @@ int md_attention_bf16(const void* qkv, void* out, int B, int L, int NH, int DH, 
 /* ---- rounding / decode ---- */
 /* get_efficient_knn (models/rounding.py:21-28): idx[m] = argmin_v clamp(|E_v|^2 + |x_m|^2 - 2 E_v.x_m, 0),
  * lowest v on ties.  x fp32 [M,D], E fp32 [V,D], idx int32 [M]; margin (optional, fp32 [M]) = second-best minus
- * best distance.  D must be a multiple of 4. */
+ * best distance.  D must be a multiple of 4.
+ * Non-finite inputs: every id written lies in [0, V).  A NaN key is clamped to 0 by the clamp above, so it ties with an
+ * exact hit (lowest v wins); md_logits_argmax never picks a NaN logit, gives a row with no logit above -inf the lowest
+ * id whose logit is -inf, and a row whose logits are all NaN id 0 (what torch.argmax gives for an all-NaN row). */
 int md_round_argmin(const float* x, const float* E, int32_t* idx, float* margin, int64_t M, int V, int D,
                     cudaStream_t stream);
 /* get_logits + argmax (models/network.py:91-93, run/sample.py:219-220): tok[m] = argmax_v (x_m.E_v + bias_v).
@@ -121,7 +124,9 @@ int md_dist_scores(const float* x, const float* dot, const float* esq, float* ou
  *     constant per row, the reference's clamp(dist, 0) only creates ties on bit-exact hits);
  *     mode 1: idx[m] = argmax_v (x_m.E_v + cst[v]), cst = lm_head bias padded with -inf  (network.py:91-93 + argmax).
  *     x2_ws: bf16 [M, 2D] scratch; with x == NULL it must already hold the [hi | lo] split of x (MD_EPI_BIAS_SPLIT) and
- *     the split pass is skipped.  Lowest index wins ties.  D must be a multiple of 64. */
+ *     the split pass is skipped.  Lowest index wins ties.  D must be a multiple of 64.
+ *     Non-finite inputs: NaN keys never win; a row with no key below +inf (any NaN / inf in x_m makes every key NaN;
+ *     in mode 1 every logit -inf or NaN) gets idx 0, so every id written lies in [0, V). */
 /* fp32 [rows, D] -> bf16 [rows, copies * 2D]: `copies` repetitions of the two-term split [hi | lo], hi = bf16(x),
  * lo = bf16(x - hi)  (operand of the split-bf16 contractions: rounding, decode, get_logits). */
 int md_split_bf16(const float* x, void* out_bf16, int64_t rows, int D, int copies, cudaStream_t stream);

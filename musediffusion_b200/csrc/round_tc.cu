@@ -6,7 +6,7 @@
 // The [V, M] distance / [M, V] logit matrix never reaches HBM: it lives in TMEM and is reduced per row in the
 // epilogue.  fp32 fidelity on bf16 tensor cores comes from splitting both operands, x = xh + xl and E = Eh + El
 // (bf16 each), and accumulating the four partial products in fp32:
-//     x.E = xh.Eh + xh.El + xl.Eh + xl.El          (relative error ~2^-17 of |x||E|, i.e. fp32-grade)
+//     x.E ~ xh.Eh + xh.El + xl.Eh + xl.El          (dropped split residuals <= 2^-15 sum_d |x_d E_d|; DESIGN.md 4.4)
 // which is ONE K = 4D contraction whose k-blocks read [xh|xl] and [Eh|El] at remapped column offsets.
 //
 // Structure = the persistent tcgen05 GEMM of gemm.cu (TMA producer warp, MMA warp, 8 epilogue warps, two TMEM
@@ -227,7 +227,8 @@ round_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 best.s = fminf(fminf(best.s, os), lose);
                 const int64_t row = (int64_t)m_blk * RT_BM + r;
                 if (row < p.M) {
-                    p.idx[row] = best.i;
+                    // no key compared below +inf (a NaN / inf row of x, or every logit -inf / NaN): id 0, as torch.argmax
+                    p.idx[row] = best.i < p.V ? best.i : 0;
                     if (p.margin != nullptr) p.margin[row] = best.s - best.b;
                 }
             }

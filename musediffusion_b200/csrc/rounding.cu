@@ -152,7 +152,7 @@ round_kernel(const float* __restrict__ x, const float* __restrict__ E, const flo
         }
         const int64_t tok = tok0 + tg * 8 + i;
         if (vg == 0 && tok < M) {
-            out_idx[tok] = best[i].i;
+            out_idx[tok] = best[i].i < V ? best[i].i : 0;      // MODE 1, every logit NaN: no key was taken, id 0
             if (out_margin != nullptr) out_margin[tok] = best[i].s - best[i].b;
         }
     }
