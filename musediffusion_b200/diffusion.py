@@ -85,8 +85,11 @@ def space_timesteps(num_timesteps, section_counts):
 
 
 def _extract_into_tensor(arr, timesteps, broadcast_shape):
-    """diffusion.py:904-917 (API parity; the kernels read the same fp32 values from constant memory)."""
-    res = torch.from_numpy(np.asarray(arr)).to(device=timesteps.device)[timesteps].float()
+    """diffusion.py:904-917 (API parity; the kernels read the same fp32 values from constant memory).  `arr` may also be
+    the table already uploaded to the timesteps' device."""
+    if not isinstance(arr, torch.Tensor):
+        arr = torch.from_numpy(np.asarray(arr)).to(device=timesteps.device)
+    res = arr[timesteps].float()
     while res.dim() < len(broadcast_shape):
         res = res[..., None]
     return res.expand(broadcast_shape)
@@ -146,7 +149,7 @@ class GaussianDiffusion:
 
     noise_source = None     # optional callable(shape, kind) -> CUDA float tensor; None = in-kernel Philox
     rounding_trace = None   # optional list: every fused rounding call appends (ids int32 [M], top-2 margin fp32 [M]) clones
-    use_cuda_graph = True   # loops of >= GRAPH_MIN_STEPS steps replay ONE captured CUDA graph of a reverse step (fused path only)
+    use_cuda_graph = True   # loops of >= GRAPH_MIN_STEPS steps replay captured CUDA graphs of the reverse step (fused path only)
     GRAPH_MIN_STEPS = 4
     seq_offset = 0          # global index of this rank's first sequence (keeps Philox noise shard-invariant)
 
@@ -290,10 +293,16 @@ class GaussianDiffusion:
         return (mean, _extract_into_tensor(self.posterior_variance, t, x_t.shape),
                 _extract_into_tensor(self.posterior_log_variance_clipped, t, x_t.shape))
 
-    def _mean_variance(self, mean, pred, t, shape):
-        """p_mean_variance's dict (diffusion.py:343-347), with the fixed-large model variance of schedule index t."""
-        return {"mean": mean, "variance": _extract_into_tensor(self.model_variance, t.long(), shape),
-                "log_variance": _extract_into_tensor(self.model_log_variance, t.long(), shape), "pred_xstart": pred}
+    def _mean_variance(self, mean, pred, t, shape, tables=None):
+        """p_mean_variance's dict (diffusion.py:343-347), with the fixed-large model variance of schedule index t.
+        `tables`: (model_variance, model_log_variance) already on t's device (`_variance_tables`)."""
+        var, log_var = tables if tables is not None else (self.model_variance, self.model_log_variance)
+        return {"mean": mean, "variance": _extract_into_tensor(var, t.long(), shape),
+                "log_variance": _extract_into_tensor(log_var, t.long(), shape), "pred_xstart": pred}
+
+    def _variance_tables(self, device):
+        """the two float64 model-variance tables on `device`, uploaded once per progressive loop instead of once per step"""
+        return tuple(torch.from_numpy(a).to(device) for a in (self.model_variance, self.model_log_variance))
 
     def p_mean_variance(self, model, x, t, clip_denoised=True, denoised_fn=None, model_kwargs=None):
         """diffusion.py:280-347: dict(mean, variance, log_variance, pred_xstart)."""
@@ -337,12 +346,13 @@ class GaussianDiffusion:
 
     def _loop(self, mode, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device, progress, top_p,
               clamp_step, clamp_first, mask, x_start, eta, indices, want_aux):
-        """Generator of (sample, pred_xstart, mean, t) per reverse step.  Our denoiser, rounding at every step, in-kernel
-        noise and a [B, L, D] state: the fused step body of `_fused_loop`, replayed as a captured CUDA graph for chains of
-        >= GRAPH_MIN_STEPS steps unless `use_cuda_graph` is off or `ops.profile_step` is timing the launches.  Everything
-        else (arbitrary callables, progressive loops, `noise_source`, `rounding_trace`, clamp gating) runs step by step
-        through `_step`; with our denoiser there the posterior kernel also emits the bf16 operand of the next step's first
-        GEMM, and the batch shares one time-embedding row (all sequences share t inside the loops, diffusion.py:516,887)."""
+        """Generator of (sample, pred_xstart, mean, t) per reverse step.  Our denoiser, in-kernel noise, a [B, L, D] state
+        and `denoised_fn` either our rounding or None: the fused step bodies of `_fused_loop` (progressive loops, clamp
+        gating and `rounding_trace` included), replayed as captured CUDA graphs for chains of >= GRAPH_MIN_STEPS steps
+        unless `use_cuda_graph` is off or `ops.profile_step` is timing the launches.  What cannot be captured (arbitrary
+        `model` / `denoised_fn` callables, `noise_source`, other state shapes) runs step by step through `_step`; with our
+        denoiser there the posterior kernel also emits the bf16 operand of the next step's first GEMM, and the batch shares
+        one time-embedding row (all sequences share t inside the loops, diffusion.py:516,887)."""
         if device is None:
             device = next(model.parameters()).device
         assert isinstance(shape, (tuple, list))
@@ -384,11 +394,11 @@ class GaussianDiffusion:
             return (i >= clamp_step) if clamp_first else not (i > clamp_step)
 
         E = rounding_weight_of(denoised_fn)
-        if (fast is not None and not want_aux and self.noise_source is None and self.rounding_trace is None and E is not None
-                and all(rounds_at(i) for i in idx_list) and x.dim() == 3):
+        if fast is not None and self.noise_source is None and (E is not None or denoised_fn is None) and x.dim() == 3:
+            rounds = [rounds_at(i) and E is not None for i in idx_list]
             capture = self.use_cuda_graph and len(idx_list) >= self.GRAPH_MIN_STEPS and ops._PROFILE[0] is None
-            yield from self._fused_loop(mode, fast, x, E, t_idx, t_model, indices, clip_denoised, top_p, mask, x_start, eta,
-                                        capture)
+            yield from self._fused_loop(mode, fast, x, E, t_idx, t_model, indices, rounds, clip_denoised, top_p, mask, x_start,
+                                        eta, want_aux, capture)
             return
         x_bf16 = None
         for k, i in enumerate(indices):
@@ -405,63 +415,94 @@ class GaussianDiffusion:
                                        want_aux=want_aux, model_output=model_output, out_bf16=x_bf16)
             yield x, pred, mean, t_arg
 
-    def _fused_loop(self, mode, fast, x, E, t_idx, t_model, indices, clip_denoised, top_p, mask, x_start, eta, capture):
-        """The chain as one fixed reverse-step body whose per-step inputs live in device memory: `md_step_advance` moves a
+    def _fused_loop(self, mode, fast, x, E, t_idx, t_model, indices, rounds, clip_denoised, top_p, mask, x_start, eta,
+                    want_aux, capture):
+        """The chain as fixed reverse-step bodies whose per-step inputs live in device memory: `md_step_advance` moves a
         cursor over the index tables and publishes the schedule index, the denoiser's timestep value and the Philox
         counter of the step, which the posterior kernel reads.  x_t is updated in place (the posterior kernel is
         elementwise) and its bf16 copy, padded to the operand width Dp with zero columns, feeds the next step's first GEMM.
-        `capture`: the first step runs eagerly (one-time set-up: shared-memory attributes, weight pack, tensor maps), the
-        second is captured as a CUDA graph (SURVEY.md section 7 step 7) and every later step replays it.  Otherwise every
-        step launches the same body directly, so per-launch timings measure the kernels a replay runs."""
+        `rounds[k]`: step k rounds to the embedding (`round_step`) or posts the model's x0 as is (`plain_step`, clamp
+        gating, diffusion.py:517-526).  Clamp gating splits a chain into at most two contiguous runs of one body.
+        `capture`: the first step of each run runs eagerly (one-time set-up: shared-memory attributes, weight pack, tensor
+        maps, workspaces), the second is captured as a CUDA graph (SURVEY.md section 7 step 7) and every later step of the
+        run replays it.  A run's graph is captured from the pool of the previous run's, which is never replayed again, so
+        every buffer one body hands to the other is allocated here, before either capture.  Otherwise every step launches
+        its body directly, so per-launch timings measure the kernels a replay runs.
+        `want_aux` (progressive loops): the posterior kernel also writes pred_xstart and the mean, and every step yields
+        clones of sample, pred_xstart and mean, which stay valid after later steps.  `rounding_trace`: the rounding kernel
+        writes its top-2 margins and every rounding step appends clones of ids and margins."""
         dev = x.device
         self._upload_schedule()
         x = x.clone()                                   # updated in place: never the caller's tensor
         pk = fast.weight_pack()
         xb = ops.cast_bf16(x, width=pk.Dp)
-        # x0-predicting model: the last Linear emits the [hi | lo] bf16 split that the rounding contraction consumes, the fp32
-        # model output never exists; an eps-predicting model needs it in fp32 for x0 = sr x_t - srm1 eps first
+        any_round, any_plain = any(rounds), not all(rounds)
+        # x0-predicting model: the last Linear of a rounding step emits the [hi | lo] bf16 split that the rounding
+        # contraction consumes, the fp32 model output never exists there; an eps-predicting model needs it in fp32 for
+        # x0 = sr x_t - srm1 eps first, and a plain step hands it to the posterior kernel
         use_split = self.predict_xstart and pk.has_down
-        mo = torch.empty_like(x) if not use_split else None
-        mo_split = torch.empty(x.shape[:-1] + (2 * pk.Dp,), dtype=torch.bfloat16, device=dev) if use_split else None
+        mo = torch.empty_like(x) if any_plain or not use_split else None
+        mo_split = torch.empty(x.shape[:-1] + (2 * pk.Dp,), dtype=torch.bfloat16, device=dev) if use_split and any_round else None
         cursor = torch.zeros(1, dtype=torch.int32, device=dev)
         t_cur = torch.zeros(1, dtype=torch.int32, device=dev)
         tm_cur = torch.zeros(1, dtype=torch.float32, device=dev)
         ctr_cur = torch.zeros(1, dtype=torch.int64, device=dev)
         ctr_base = self._noise_calls + 1                # the value _next_counter() hands to the first step of an eager loop
         seed = self._seed()
-        se = ops.split_embedding(E)
-        # clip_denoised after rounding = gathering rows of clamp(E, -1, 1): built once per embedding matrix, not per token and step
-        E_step, clip_step = (se.E_clamped, 2) if clip_denoised else (E, 0)
-        idx = torch.empty((x.shape[0] * x.shape[1],), dtype=torch.int32, device=dev)
+        M = x.shape[0] * x.shape[1]
+        idx = torch.empty((M,), dtype=torch.int32, device=dev)
+        trace = self.rounding_trace if any_round else None
+        margin = torch.empty((M,), dtype=torch.float32, device=dev) if trace is not None else None
+        pred_out = torch.empty_like(x) if want_aux else None
+        mean_out = torch.empty_like(x) if want_aux else None
+        if any_round:
+            se = ops.split_embedding(E)
+            # clip_denoised after rounding = gathering rows of clamp(E, -1, 1): built once per embedding matrix, not per
+            # token and step
+            E_step, clip_step = (se.E_clamped, 2) if clip_denoised else (E, 0)
         _, tp = _noise_kind(mode, top_p)
+        post = dict(seed=seed, seq_offset=self.seq_offset, mask=mask, x_start=x_start, eta=eta, top_p=tp, out=x, out_bf16=xb,
+                    pred_out=pred_out, mean_out=mean_out, step_counter_dev=ctr_cur)
 
-        def one_step():
+        def model_x0():
+            out = fast.denoise(x, tm_cur, x_bf16=xb, uniform_t=True, out=mo)
+            return out if self.predict_xstart else ops.xstart_from_eps(x, out, t_cur)
+
+        def round_step():
             ops.step_advance(cursor, t_idx, t_model, t_cur, tm_cur, ctr_cur, ctr_base)
             if use_split:
                 fast.denoise(x, tm_cur, x_bf16=xb, uniform_t=True, split_out=mo_split)
-                ops.round_argmin_tc(None, se, out=idx, presplit=mo_split)
+                ops.round_argmin_tc(None, se, out=idx, presplit=mo_split, margin_out=margin)
             else:
-                out = fast.denoise(x, tm_cur, x_bf16=xb, uniform_t=True, out=mo)
-                if not self.predict_xstart:
-                    out = ops.xstart_from_eps(x, out, t_cur)
-                ops.round_argmin_tc(out, se, out=idx)
-            ops.posterior_step(x, t_cur, mode, idx=idx, E=E_step, seed=seed, seq_offset=self.seq_offset, mask=mask, x_start=x_start,
-                               eta=eta, clip=clip_step, top_p=tp, out=x, out_bf16=xb, step_counter_dev=ctr_cur)
+                ops.round_argmin_tc(model_x0(), se, out=idx, margin_out=margin)
+            ops.posterior_step(x, t_cur, mode, idx=idx, E=E_step, clip=clip_step, **post)
+
+        def plain_step():
+            ops.step_advance(cursor, t_idx, t_model, t_cur, tm_cur, ctr_cur, ctr_base)
+            ops.posterior_step(x, t_cur, mode, pred=model_x0(), clip=clip_denoised, **post)
 
         graph, nodes = None, 0
         for k, i in enumerate(indices):
-            if k == 0 or not capture:
-                one_step()
+            body = round_step if rounds[k] else plain_step
+            run_start = k == 0 or rounds[k] != rounds[k - 1]
+            if run_start or not capture:
+                graph = None
+                body()
             else:
                 if graph is None:
                     before = ops.launch_count()
-                    graph = _capture(dev, one_step)
+                    graph = _capture(dev, body)
                     nodes = ops.launch_count() - before          # kernels recorded by the capture (nothing ran yet)
                     ops.add_launches(-nodes)
                 graph.replay()
                 ops.add_launches(nodes)
             self._noise_calls += 1
-            yield x, None, None, t_idx[k:k + 1]
+            if trace is not None and rounds[k]:
+                trace.append((idx.clone(), margin.clone()))
+            if want_aux:
+                yield x.clone(), pred_out.clone(), mean_out.clone(), t_idx[k:k + 1]
+            else:
+                yield x, None, None, t_idx[k:k + 1]
 
     def p_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, model_kwargs=None,
                       device=None, progress=False, top_p=None, clamp_step=None, clamp_first=None, mask=None,
@@ -477,11 +518,14 @@ class GaussianDiffusion:
                                   clamp_first=None, mask=None, x_start=None, eta=0.0, t_enc=None):
         """diffusion.py:475-540: generator of p_sample dicts."""
         indices = list(range(self.num_timesteps))[::-1][slice(t_enc)]
+        tables = None
         for sample, pred, mean, t in self._loop(_lib.STEP_DDPM, model, shape, noise, clip_denoised, denoised_fn,
                                                 model_kwargs, device, progress, top_p, clamp_step, clamp_first, mask,
                                                 x_start, eta, indices, want_aux=True):
+            if tables is None:
+                tables = self._variance_tables(t.device)
             yield {"sample": sample, "pred_xstart": pred, "greedy_mean": mean,
-                   "out": self._mean_variance(mean, pred, t, sample.shape)}
+                   "out": self._mean_variance(mean, pred, t, sample.shape, tables)}
 
     def ddim_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, model_kwargs=None,
                          device=None, progress=False, top_p=None, clamp_step=None, clamp_first=None, mask=None,

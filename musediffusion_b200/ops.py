@@ -278,10 +278,11 @@ def split_embedding(E):
     return hit[0]
 
 
-def round_argmin_tc(x, se, cst=None, mode=0, want_margin=False, out=None, presplit=None):
+def round_argmin_tc(x, se, cst=None, mode=0, want_margin=False, out=None, presplit=None, margin_out=None):
     """tensor-core nearest-embedding ids (mode 0, cst = |E|^2) or argmax-logit ids (mode 1, cst = padded bias).
     x: fp32 [..., D].  `presplit`: bf16 [M, 2Dp] = [hi | 0 | lo | 0] of x already written by the producing GEMM
-    (EPI_BIAS_SPLIT with N = Dp); x is then ignored."""
+    (EPI_BIAS_SPLIT with N = Dp); x is then ignored.  `margin_out`: fp32 [M] that receives the top-2 margins (as
+    want_margin does, into a buffer the caller owns)."""
     if presplit is not None:
         assert presplit.dtype == BF16 and presplit.is_contiguous() and presplit.shape[-1] == 2 * se.Dp
         M = presplit.numel() // (2 * se.Dp)
@@ -291,8 +292,10 @@ def round_argmin_tc(x, se, cst=None, mode=0, want_margin=False, out=None, prespl
         M = x.numel() // se.D
         ws, dev = se.workspace(M), x.device
     idx = out if out is not None else torch.empty((M,), dtype=torch.int32, device=dev)
-    margin = torch.empty((M,), dtype=torch.float32, device=dev) if want_margin else None
-    _cu(x, ws)
+    if margin_out is not None:
+        assert margin_out.dtype == torch.float32 and margin_out.is_contiguous() and margin_out.numel() == M
+    margin = margin_out if margin_out is not None else (torch.empty((M,), dtype=torch.float32, device=dev) if want_margin else None)
+    _cu(x, ws, margin)
     cst = se.sqnorm if cst is None else cst
     if se.Dp == se.D:
         K.round_argmin_tc(x, se.E2, cst, ws, idx, margin, se.V, mode)
