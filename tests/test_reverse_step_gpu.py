@@ -354,9 +354,9 @@ CHAINS = {
 }
 
 
-def _chain_config(name):
+def _chain_config(chain):
     c = dict(strength=1.0, top_p=0, eta=0.0, clip=True, pxs=True, rows=None, seq_offset=0)
-    c.update(CHAINS[name])
+    c.update(chain)
     if c["rows"] is not None:
         c["seq_offset"] = c["rows"].start
     return SimpleNamespace(**c)
@@ -413,7 +413,12 @@ def test_fused_loop_matches_oracle_through_per_step_path(name):
     rounding call traced) agrees with it under the parity rule.  3. The production loop (in-kernel noise, no trace), graph-
     replayed and eager, reproduces the per-step path's final sample and decoded tokens bit for bit and counts the same noise
     calls: step advance, counter base, pre-clamped embedding, split epilogue and in-kernel noise are those of step 2."""
-    c = _chain_config(name)
+    _check_chain(name, CHAINS[name])
+
+
+def _check_chain(name, chain):
+    """the three steps of test_fused_loop_matches_oracle_through_per_step_path for one CHAINS-style entry"""
+    c = _chain_config(chain)
     seed = 1000 + sum(map(ord, name))
     torch.manual_seed(seed)
     p = O.make_random_params(seed=seed % 997, seq_len=c.L, hidden_dim=c.D)

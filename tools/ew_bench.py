@@ -50,7 +50,14 @@ rep("  ... gathering pre-clamped rows (the loop's path)", ms, M * (512 + 4 + 512
 ms = timeit(lambda: ops.posterior_step(x, t, _lib.STEP_DDPM, idx=idx, E=E, noise=noise, mask=mask, x_start=xs, out=out, out_bf16=xb))
 rep("posterior DDPM external noise", ms, M * (512 + 4 + 512 + 512 + 256))
 ms = timeit(lambda: ops.posterior_step(x, t, _lib.STEP_DDIM, idx=idx, E=E, seed=1, step_counter=3, mask=mask, x_start=xs, out=out, out_bf16=xb))
-rep("posterior DDIM philox untruncated", ms, M * (512 + 4 + 512 + 256))
+rep("posterior DDIM eta=0 (sigma 0: no draws)", ms, M * (512 + 4 + 512 + 256))
+# the general quantile (top_p = 0 or > 1): DDPM with top_p > 1, DDIM with eta > 0, the generation-mode initial noise
+ms = timeit(lambda: ops.posterior_step(x, t, _lib.STEP_DDPM, idx=idx, E=E, seed=1, step_counter=3, mask=mask, x_start=xs, top_p=2.0, out=out, out_bf16=xb))
+rep("posterior DDPM philox top_p=2 (general)", ms, M * (512 + 4 + 512 + 256))
+ms = timeit(lambda: ops.posterior_step(x, t, _lib.STEP_DDIM, idx=idx, E=E, seed=1, step_counter=3, mask=mask, x_start=xs, eta=0.5, out=out, out_bf16=xb))
+rep("posterior DDIM philox eta=0.5 (general)", ms, M * (512 + 4 + 512 + 256))
+ms = timeit(lambda: ops.fill_normal((B, L, D), dev, seed=1, step_counter=3))
+rep("fill_normal untruncated (general)", ms, M * D * 4)
 ms = timeit(lambda: ops.layernorm(h, g, bt, 1e-12, resid=r, out=ho))
 rep("layernorm(x + resid) bf16", ms, M * H * 2 * 3)
 ms = timeit(lambda: ops.round_argmin(x, E))
