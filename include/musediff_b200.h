@@ -174,6 +174,22 @@ int md_posterior_step_ld(const float* x_t, const int32_t* idx, const float* pred
                          const int32_t* mask, int64_t mask_tok_stride, int64_t mask_d_stride, const float* x_start,
                          float* x_out, void* out_bf16, int bf16_ld, float* pred_out, float* mean_out, int B, int L, int D,
                          int mode, float eta, int clip, float top_p, const uint64_t* step_counter_dev, cudaStream_t stream);
+/* ---- one step of the DPM-Solver++(2M) sampler (Lu et al., "DPM-Solver++", 2022, Algorithm 2: multistep, second order,
+ * data prediction) — an addition beyond the reference, which samples with DDPM / DDIM only ----
+ *   p    = idx ? E[idx] : pred_in, clipped as in md_posterior_step (clip 0 / 1 / 2 with the same meaning)
+ *   (a, b, c0, c1) = coef[row]: row = *cursor - 1 clamped to [0, n_coef - 1] (the cursor as md_step_advance leaves it, so one
+ *        captured graph serves every step), or row 0 when cursor is NULL (then n_coef must be 1)
+ *   d    = c1 != 0 ? c0 p + c1 q : c0 p,  q = pred_hist[m, d] (the previous evaluation's p; never read where c1 == 0)
+ *   pred_hist[m, d] = p                   (in place, after the read)
+ *   x'   = a != 0 ? a x_t + b d : b d     (x_t is not read where a == 0: the row (0, 1, 1, 0) writes p itself)
+ *   x'   = mask == 0 ? x_start : x'       (mask as md_posterior_step)
+ * fp32, every product and sum rounded separately (no FMA contraction).  x_out may alias x_t; out_bf16 (optional) = bf16
+ * copy of x' in rows of stride bf16_ld >= D (a multiple of 4), columns D..bf16_ld-1 never written.  pred_hist fp32 [M, D],
+ * coef fp32 [n_coef, 4].  D must be a multiple of 4.  The step draws no noise. */
+int md_dpm_solver_step(const float* x_t, const int32_t* idx, const float* pred_in, const float* E, float* pred_hist,
+                       const float* coef, int n_coef, const int32_t* cursor, const int32_t* mask, int64_t mask_tok_stride,
+                       int64_t mask_d_stride, const float* x_start, float* x_out, void* out_bf16, int bf16_ld, int B, int L,
+                       int D, int clip, cudaStream_t stream);
 /* Loop state on the device, so that ONE captured CUDA graph of a reverse step can be replayed for every index of the
  * loops diffusion.py:508-540 / :878-901 (the reference rebuilds t = th.tensor([i] * B) on the host every iteration):
  * k = *cursor; *t_cur = t_idx[k]; *tm_cur = t_model[k] (the value _WrappedModel feeds the denoiser, :1027-1032);

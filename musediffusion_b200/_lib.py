@@ -41,6 +41,8 @@ SIGNATURES = {
     "md_posterior_step_ld": [c_p, c_p, c_p, c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_p,
                              c_i, c_p, c_p, c_i, c_i, c_i, c_i, c_f, c_i, c_f, c_p, c_p],
     "md_step_advance": [c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_u64, c_p],
+    "md_dpm_solver_step": [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i64, c_i64, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i,
+                           c_p],
     "md_xstart_from_eps": [c_p, c_p, c_p, c_i, c_p, c_i, c_i, c_i, c_p],
     "md_q_sample": [c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_i, c_i, c_i, c_p],
     "md_q_sample_ld": [c_p, c_p, c_u64, c_u64, c_i64, c_p, c_i, c_p, c_i64, c_i64, c_p, c_p, c_i, c_i, c_i, c_i, c_p],

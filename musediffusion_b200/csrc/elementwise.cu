@@ -438,6 +438,115 @@ xstart_from_eps_kernel(const float* x_t, const float* eps, const int32_t* t, int
     }
 }
 
+// ----------------------------------------------------------------------------------------------
+// DPM-Solver++(2M) step (Lu et al., "DPM-Solver++", Algorithm 2): x' = a x + b (c0 p + c1 q), q = x0 of the previous
+// evaluation read from (and p written back to) the history buffer in place
+// ----------------------------------------------------------------------------------------------
+struct DpmArgs {
+    const float* x_t;
+    const int32_t* idx;
+    const float* pred_in;
+    const float* E;
+    float* hist;
+    const float* coef;       // [n_coef, 4] = (a, b, c0, c1)
+    const int32_t* cursor;   // optional: row *cursor - 1 (after md_step_advance), clamped to [0, n_coef - 1]
+    int n_coef;
+    const int32_t* mask;
+    int64_t mask_tok_stride, mask_d_stride;
+    const float* x_start;
+    float* x_out;
+    __nv_bfloat16* out_bf16;
+    int B, L, D, vshift;
+    int bf16_ld;
+    int clip;
+};
+// Same load / gather / arithmetic phases as posterior_step_kernel: kStepUnroll float4 items in flight per thread, every
+// load of a group issued before any store.  x_t is not read where a == 0 and the history not where c1 == 0.
+template <typename IdxT>
+__global__ void __launch_bounds__(256) dpm_solver_step_kernel(const DpmArgs a) {
+    int row = 0;
+    if (a.cursor != nullptr) row = min(max(*a.cursor - 1, 0), a.n_coef - 1);
+    const float4 c = *reinterpret_cast<const float4*>(a.coef + 4 * row);
+    const float ca = c.x, cb = c.y, c0 = c.z, c1 = c.w;
+    const int vec_per_tok = a.D >> 2;
+    const IdxT total = (IdxT)((int64_t)a.B * a.L * vec_per_tok);
+    const IdxT nthreads = (IdxT)gridDim.x * (IdxT)blockDim.x;
+    for (IdxT i0 = (IdxT)blockIdx.x * (IdxT)blockDim.x + (IdxT)threadIdx.x; i0 < total; i0 += nthreads * kStepUnroll) {
+        IdxT off[kStepUnroll], tok[kStepUnroll];
+        int dd[kStepUnroll];
+        bool ok[kStepUnroll];
+        float4 x[kStepUnroll], p[kStepUnroll], q[kStepUnroll];
+        int32_t id[kStepUnroll], mk[kStepUnroll];
+#pragma unroll
+        for (int u = 0; u < kStepUnroll; ++u) {
+            const IdxT i = i0 + (IdxT)u * nthreads;
+            ok[u] = i < total;
+            const TokPos tp = tok_pos(ok[u] ? (int64_t)i : 0, vec_per_tok, a.vshift, a.L);
+            tok[u] = (IdxT)tp.tok; dd[u] = tp.d;
+            off[u] = (IdxT)tp.tok * (IdxT)a.D + (IdxT)tp.d;
+            if (ok[u]) {
+                if (ca != 0.0f) x[u] = ld_stream_f4(a.x_t + off[u]);
+                if (c1 != 0.0f) q[u] = ld_stream_f4(a.hist + off[u]);
+                if (a.idx != nullptr) id[u] = a.idx[tok[u]];
+                else p[u] = ld_stream_f4(a.pred_in + off[u]);
+                mk[u] = (a.mask != nullptr && a.mask_d_stride == 0) ? a.mask[tok[u] * a.mask_tok_stride] : 1;
+            }
+        }
+        if (a.idx != nullptr) {
+#pragma unroll
+            for (int u = 0; u < kStepUnroll; ++u)
+                if (ok[u]) p[u] = *reinterpret_cast<const float4*>(a.E + (int64_t)id[u] * a.D + dd[u]);
+        }
+#pragma unroll
+        for (int u = 0; u < kStepUnroll; ++u) {
+            if (!ok[u]) continue;
+            float4 pp = p[u];
+            pp.x = clampf(pp.x, a.clip); pp.y = clampf(pp.y, a.clip); pp.z = clampf(pp.z, a.clip); pp.w = clampf(pp.w, a.clip);
+            // first-order rows (c1 == 0) never read the history: a fresh buffer may hold NaN, and 0 * NaN = NaN
+            float4 d;
+            if (c1 != 0.0f) {
+                d.x = __fadd_rn(__fmul_rn(c0, pp.x), __fmul_rn(c1, q[u].x));
+                d.y = __fadd_rn(__fmul_rn(c0, pp.y), __fmul_rn(c1, q[u].y));
+                d.z = __fadd_rn(__fmul_rn(c0, pp.z), __fmul_rn(c1, q[u].z));
+                d.w = __fadd_rn(__fmul_rn(c0, pp.w), __fmul_rn(c1, q[u].w));
+            } else {
+                d = make_float4(__fmul_rn(c0, pp.x), __fmul_rn(c0, pp.y), __fmul_rn(c0, pp.z), __fmul_rn(c0, pp.w));
+            }
+            st_stream_f4(a.hist + off[u], pp);
+            // a == 0 (the step to clean data): the output is b d, which is p itself for the row (0, 1, 1, 0)
+            float4 o;
+            if (ca != 0.0f) {
+                o.x = __fadd_rn(__fmul_rn(ca, x[u].x), __fmul_rn(cb, d.x));
+                o.y = __fadd_rn(__fmul_rn(ca, x[u].y), __fmul_rn(cb, d.y));
+                o.z = __fadd_rn(__fmul_rn(ca, x[u].z), __fmul_rn(cb, d.z));
+                o.w = __fadd_rn(__fmul_rn(ca, x[u].w), __fmul_rn(cb, d.w));
+            } else {
+                o = make_float4(__fmul_rn(cb, d.x), __fmul_rn(cb, d.y), __fmul_rn(cb, d.z), __fmul_rn(cb, d.w));
+            }
+            if (a.mask != nullptr) {
+                if (a.mask_d_stride == 0) {
+                    if (mk[u] == 0) o = *reinterpret_cast<const float4*>(a.x_start + off[u]);
+                } else {
+                    const int32_t* mp = a.mask + tok[u] * a.mask_tok_stride + (int64_t)dd[u] * a.mask_d_stride;
+                    const int64_t ds = a.mask_d_stride;
+                    const bool k0 = mp[0] == 0, k1 = mp[ds] == 0, k2 = mp[2 * ds] == 0, k3 = mp[3 * ds] == 0;
+                    if (k0 | k1 | k2 | k3) {
+                        const float4 xs = *reinterpret_cast<const float4*>(a.x_start + off[u]);
+                        if (k0) o.x = xs.x;
+                        if (k1) o.y = xs.y;
+                        if (k2) o.z = xs.z;
+                        if (k3) o.w = xs.w;
+                    }
+                }
+            }
+            st_stream_f4(a.x_out + off[u], o);
+            if (a.out_bf16 != nullptr)
+                *reinterpret_cast<uint2*>(a.out_bf16 + tok[u] * (IdxT)a.bf16_ld + (IdxT)dd[u]) =
+                    make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
+        }
+    }
+}
+
 struct QSampleArgs {
     const float* x0;
     const float* noise;
@@ -934,6 +1043,37 @@ extern "C" __attribute__((visibility("default"))) int md_posterior_step(const fl
     return md_posterior_step_ld(x_t, idx, pred_in, E, noise, seed, step_counter, seq_offset, t, t_stride, mask, mask_tok_stride,
                                 mask_d_stride, x_start, x_out, out_bf16, D, pred_out, mean_out, B, L, D, mode, eta, clip, top_p,
                                 step_counter_dev, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int md_dpm_solver_step(const float* x_t, const int32_t* idx, const float* pred_in, const float* E,
+                                  float* pred_hist, const float* coef, int n_coef, const int32_t* cursor,
+                                  const int32_t* mask, int64_t mask_tok_stride, int64_t mask_d_stride, const float* x_start,
+                                  float* x_out, void* out_bf16, int bf16_ld, int B, int L, int D, int clip,
+                                  cudaStream_t stream) {
+    if (D <= 0 || D % 4 != 0) { set_last_error("md_dpm_solver_step: D=%d must be a positive multiple of 4", D); return MD_ERR_ARG; }
+    if (bf16_ld < D || bf16_ld % 4 != 0) { set_last_error("md_dpm_solver_step: bf16_ld=%d must be a multiple of 4 >= D=%d", bf16_ld, D); return MD_ERR_ARG; }
+    if ((idx == nullptr) == (pred_in == nullptr)) { set_last_error("md_dpm_solver_step: exactly one of idx / pred_in"); return MD_ERR_ARG; }
+    if (idx != nullptr && E == nullptr) { set_last_error("md_dpm_solver_step: idx needs E"); return MD_ERR_ARG; }
+    if (clip == 2 && idx == nullptr) { set_last_error("md_dpm_solver_step: clip = 2 (pre-clamped E) needs idx"); return MD_ERR_ARG; }
+    if (clip < 0 || clip > 2) { set_last_error("md_dpm_solver_step: bad clip %d", clip); return MD_ERR_ARG; }
+    if (mask != nullptr && x_start == nullptr) { set_last_error("md_dpm_solver_step: mask needs x_start"); return MD_ERR_ARG; }
+    if (pred_hist == nullptr || coef == nullptr || n_coef <= 0 || (cursor == nullptr && n_coef != 1)) {
+        set_last_error("md_dpm_solver_step: history and coefficient table required; without a cursor the table has one row (n_coef=%d)", n_coef);
+        return MD_ERR_ARG;
+    }
+    if ((int64_t)B * L == 0) return MD_OK;
+    if ((int64_t)B * L >= (int64_t)1 << 31) { set_last_error("md_dpm_solver_step: more than 2^31 tokens"); return MD_ERR_ARG; }
+    DpmArgs a;
+    a.x_t = x_t; a.idx = idx; a.pred_in = pred_in; a.E = E; a.hist = pred_hist; a.coef = coef; a.cursor = cursor; a.n_coef = n_coef;
+    a.mask = mask; a.mask_tok_stride = mask_tok_stride; a.mask_d_stride = mask_d_stride; a.x_start = x_start; a.x_out = x_out;
+    a.out_bf16 = reinterpret_cast<__nv_bfloat16*>(out_bf16); a.B = B; a.L = L; a.D = D; a.vshift = vec_shift(D);
+    a.bf16_ld = bf16_ld; a.clip = clip;
+    const int grid = ew_grid(((int64_t)B * L * (D / 4) + kStepUnroll - 1) / kStepUnroll, 256);
+    if ((int64_t)B * L * bf16_ld + (int64_t)grid * 256 * kStepUnroll * 4 < ((int64_t)1 << 31))
+        dpm_solver_step_kernel<int32_t><<<grid, 256, 0, stream>>>(a);
+    else
+        dpm_solver_step_kernel<int64_t><<<grid, 256, 0, stream>>>(a);
+    return check_cuda(cudaGetLastError(), "dpm_solver_step launch");
 }
 
 extern "C" __attribute__((visibility("default"))) int md_xstart_from_eps(const float* x_t, const float* eps, const int32_t* t, int t_stride, float* out, int B, int L,

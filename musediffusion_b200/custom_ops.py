@@ -186,6 +186,13 @@ def _step_advance(cursor, t_idx, t_model, t_cur, tm_cur, ctr_cur, ctr_base):
            _stream())
 
 
+def _dpm_solver_step(x_t, idx, pred, E, pred_hist, coef, cursor, mask, mask_tok_stride, mask_d_stride, x_start, out, out_bf16, clip):
+    B, L, D = x_t.shape
+    launch("md_dpm_solver_step", _p(x_t), _p(idx), _p(pred), _p(E), _p(pred_hist), _p(coef), coef.shape[0], _p(cursor), _p(mask),
+           mask_tok_stride, mask_d_stride, _p(x_start), _p(out), _p(out_bf16), out_bf16.shape[-1] if out_bf16 is not None else D,
+           B, L, D, int(clip), _stream())
+
+
 # ------------------------------------------------------------------------------------------------ rows either side of the path
 def _decode_prepare(tokens, mask, strict, status, note_len, notes, meta):
     B, L = tokens.shape
@@ -246,6 +253,9 @@ _define("q_sample_ld(Tensor x0, Tensor? noise, int seed, int step_counter, int s
 _define("fill_normal(Tensor(a!) out, int seed, int step_counter, int elem_offset, float top_p) -> ()", _fill_normal)
 _define("step_advance(Tensor(a!) cursor, Tensor t_idx, Tensor t_model, Tensor(b!) t_cur, Tensor(c!) tm_cur, Tensor(d!) ctr_cur, "
         "int ctr_base) -> ()", _step_advance)
+_define("dpm_solver_step(Tensor x_t, Tensor? idx, Tensor? pred, Tensor? E, Tensor(a!) pred_hist, Tensor coef, Tensor? cursor, "
+        "Tensor? mask, int mask_tok_stride, int mask_d_stride, Tensor? x_start, Tensor(b!) out, Tensor(c!)? out_bf16, int clip) -> ()",
+        _dpm_solver_step)
 _define("decode_prepare(Tensor tokens, Tensor mask, bool strict, Tensor(a!) status, Tensor(b!) note_len, Tensor(c!) notes, "
         "Tensor(d!) meta) -> ()", _decode_prepare)
 _define("merge_and_mask(Tensor? src, Tensor src_len, Tensor trg, Tensor trg_len, int seq_len, int end_token, Tensor(a!) input_ids, "
@@ -257,6 +267,6 @@ _define("onnc(Tensor vectors, Tensor(a!)? msim, Tensor(b!) most_sim) -> ()", _on
 OP_NAMES = ["cast_f32_bf16", "cast_f32_bf16_ld", "cast_bf16_f32", "add_pos_time", "embed_gather", "timestep_mlp", "layernorm_bf16",
             "linear_bf16", "linear_bf16_cols", "attention_bf16", "round_argmin", "logits_argmax", "split_bf16", "dist_scores",
             "embed_split", "embed_split_padded", "round_argmin_tc", "round_argmin_tc_padded", "posterior_step", "posterior_step_ld",
-            "xstart_from_eps", "q_sample", "q_sample_ld", "fill_normal", "step_advance", "decode_prepare", "merge_and_mask",
-            "sequence_metrics", "onnc"]
+            "xstart_from_eps", "q_sample", "q_sample_ld", "fill_normal", "step_advance", "dpm_solver_step", "decode_prepare",
+            "merge_and_mask", "sequence_metrics", "onnc"]
 ops = getattr(torch.ops, NAMESPACE)

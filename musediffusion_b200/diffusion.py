@@ -9,6 +9,7 @@ What is mirrored (reference file:line):
   p_sample_loop(_progressive)                             :406-540
   ddim_sample / ddim_sample_loop(_progressive)            :701-757, :797-901
   space_timesteps / SpacedDiffusion / _WrappedModel       :920-1032
+Beyond the reference: dpm_solver_sample_loop, the DPM-Solver++(2M) sampler (md_dpm_solver_step) for tens of evaluations.
 Training losses (:187-192, :542-699) are out of scope (SURVEY.md section 8) and raise NotImplementedError.
 
 Noise.  The reference draws `torch.randn_like` every step (plus a host-synchronising rejection loop for top_p).
@@ -144,6 +145,59 @@ def _collect(steps, only_last):
     return final
 
 
+def _log_snr(alphas_cumprod):
+    """lambda_i = log alpha_i - log sigma_i of every index, alpha_i = sqrt(abar_i), sigma_i = sqrt(1 - abar_i) (float64)."""
+    ab = np.asarray(alphas_cumprod, dtype=np.float64)
+    return 0.5 * np.log(ab) - 0.5 * np.log1p(-ab)
+
+
+def dpm_solver_indices(alphas_cumprod, t_start, steps):
+    """The `steps` evaluation indices of dpm_solver_sample_loop: t_start = s_0 > s_1 > ... > s_{N-1} = 0 (N = 1: [t_start]).
+    The targets are uniform in lambda: g_k is the fractional index whose lambda (interpolated in the table) is the k-th of N
+    evenly spaced values from lambda[t_start] to lambda[0]; s_k = clip(round(g_k), N - 1 - k, s_{k-1} - 1) keeps the N
+    indices distinct."""
+    T = len(alphas_cumprod)
+    t_start, steps = int(t_start), int(steps)
+    if not 0 <= t_start < T:
+        raise ValueError("t_start=%d outside the schedule's %d indices" % (t_start, T))
+    if not 1 <= steps <= t_start + 1:
+        raise ValueError("steps=%d: DPM-Solver++ needs 1 <= steps <= t_start + 1 = %d" % (steps, t_start + 1))
+    lam = _log_snr(alphas_cumprod)[:t_start + 1]
+    grid = np.arange(t_start + 1, dtype=np.float64)
+    g = np.interp(np.linspace(lam[t_start], lam[0], steps), lam[::-1], grid[::-1])     # lambda decreases with the index
+    s = [t_start]
+    for k in range(1, steps):
+        s.append(int(min(max(np.rint(g[k]), steps - 1 - k), s[-1] - 1)))
+    return s
+
+
+def dpm_solver_coefficients(alphas_cumprod, indices, order):
+    """float64 [N, 4] rows (a, b, c0, c1) of md_dpm_solver_step for the evaluation indices (DPM-Solver++(2M), Lu et al. 2022,
+    Algorithm 2).  Step k < N - 1 goes from c = s_k to n = s_{k+1}, h = lambda_n - lambda_c: a = sigma_n / sigma_c,
+    b = -alpha_n expm1(-h); the first step (and every step at order 1) uses D = x0_k (c0 = 1, c1 = 0), later ones
+    D = (1 + 1/(2r)) x0_k - 1/(2r) x0_{k-1} with r = h_{k-1} / h.  The last row (0, 1, 1, 0) returns x0_{N-1} itself."""
+    if order not in (1, 2):
+        raise ValueError("DPM-Solver++ order must be 1 or 2, got %r" % (order,))
+    ab = np.asarray(alphas_cumprod, dtype=np.float64)
+    lam = _log_snr(ab)
+    alpha, sigma = np.sqrt(ab), np.sqrt(1.0 - ab)
+    rows, h_prev = [], None
+    for k in range(len(indices)):
+        if k == len(indices) - 1:
+            rows.append((0.0, 1.0, 1.0, 0.0))
+            break
+        c, n = indices[k], indices[k + 1]
+        h = lam[n] - lam[c]
+        a, b = sigma[n] / sigma[c], -alpha[n] * np.expm1(-h)
+        if order == 1 or h_prev is None:
+            rows.append((a, b, 1.0, 0.0))
+        else:
+            r = h_prev / h
+            rows.append((a, b, 1.0 + 1.0 / (2.0 * r), -1.0 / (2.0 * r)))
+        h_prev = h
+    return np.array(rows, dtype=np.float64).reshape(-1, 4)
+
+
 class GaussianDiffusion:
     """Sampling utilities with the reference's attribute and method names (diffusion.py:121-901)."""
 
@@ -258,6 +312,23 @@ class GaussianDiffusion:
         assert t.numel() in (1, B)
         if model_output is None:
             model_output = self._call_model(model, x, t, model_kwargs)
+        E, idx, pred = self._processed_x0(x, t, model_output, denoised_fn)
+        kind, tp = _noise_kind(mode, top_p)
+        if noise is None:
+            noise = self._external_noise(x.shape, kind, x.device)
+        pred_out = torch.empty_like(x, dtype=torch.float32) if want_aux else None
+        mean_out = torch.empty_like(x, dtype=torch.float32) if want_aux else None
+        sample = ops.posterior_step(
+            x, t, mode, idx=idx, pred=pred, E=E, noise=noise, seed=self._seed(), step_counter=self._next_counter(),
+            seq_offset=self.seq_offset, mask=mask, x_start=x_start, eta=eta, clip=clip_denoised, top_p=tp, out_bf16=out_bf16,
+            pred_out=pred_out, mean_out=mean_out)
+        return sample, pred_out, mean_out
+
+    def _processed_x0(self, x, t, model_output, denoised_fn):
+        """x0 of one step as the posterior / DPM kernels take it -> (E, idx, pred): the model output (through
+        xstart_from_eps for an eps-predicting model), then rounded (ids into E, gathered by the kernel) when `denoised_fn`
+        is our rounding callback, or passed through an arbitrary `denoised_fn`; the kernels clip after that."""
+        B = x.shape[0]
         if not self.predict_xstart:
             model_output = ops.xstart_from_eps(x, model_output, t)
         E = rounding_weight_of(denoised_fn)
@@ -273,16 +344,7 @@ class GaussianDiffusion:
             pred = denoised_fn(model_output, t if t.numel() == B else t.expand(B))   # arbitrary user callable
         else:
             pred = model_output
-        kind, tp = _noise_kind(mode, top_p)
-        if noise is None:
-            noise = self._external_noise(x.shape, kind, x.device)
-        pred_out = torch.empty_like(x, dtype=torch.float32) if want_aux else None
-        mean_out = torch.empty_like(x, dtype=torch.float32) if want_aux else None
-        sample = ops.posterior_step(
-            x, t, mode, idx=idx, pred=pred, E=E, noise=noise, seed=self._seed(), step_counter=self._next_counter(),
-            seq_offset=self.seq_offset, mask=mask, x_start=x_start, eta=eta, clip=clip_denoised, top_p=tp, out_bf16=out_bf16,
-            pred_out=pred_out, mean_out=mean_out)
-        return sample, pred_out, mean_out
+        return E, idx, pred
 
     def q_posterior_mean_variance(self, x_start, x_t, t):
         """diffusion.py:257-278."""
@@ -344,15 +406,9 @@ class GaussianDiffusion:
         inner = model.model if isinstance(model, _WrappedModel) else model
         return inner if isinstance(inner, TransformerNetModel) else None
 
-    def _loop(self, mode, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device, progress, top_p,
-              clamp_step, clamp_first, mask, x_start, eta, indices, want_aux):
-        """Generator of (sample, pred_xstart, mean, t) per reverse step.  Our denoiser, in-kernel noise, a [B, L, D] state
-        and `denoised_fn` either our rounding or None: the fused step bodies of `_fused_loop` (progressive loops, clamp
-        gating and `rounding_trace` included), replayed as captured CUDA graphs for chains of >= GRAPH_MIN_STEPS steps
-        unless `use_cuda_graph` is off or `ops.profile_step` is timing the launches.  What cannot be captured (arbitrary
-        `model` / `denoised_fn` callables, `noise_source`, other state shapes) runs step by step through `_step`; with our
-        denoiser there the posterior kernel also emits the bf16 operand of the next step's first GEMM, and the batch shares
-        one time-embedding row (all sequences share t inside the loops, diffusion.py:516,887)."""
+    def _loop_inputs(self, model, shape, noise, device, mask, x_start):
+        """-> (device, x, mask, x_start) of a loop: the starting state (`noise`, else `noise_source`, else a Philox draw keyed by
+        the next noise counter), and the mask and x_start converted once so that the per-step kernel calls allocate nothing."""
         if device is None:
             device = next(model.parameters()).device
         assert isinstance(shape, (tuple, list))
@@ -363,12 +419,8 @@ class GaussianDiffusion:
             if x is None:
                 x = ops.fill_normal(tuple(shape), device, seed=self._seed(), step_counter=self._next_counter(),
                                     elem_offset=self.seq_offset * int(np.prod(shape[1:])))
-        fast = self._fast_model(model)
-        B = shape[0]
-        if len(indices) == 0:
-            return
         if mask is not None:
-            # convert the (usually int64, stride-0 expanded) mask ONCE so the per-step kernel call allocates nothing
+            # the (usually int64, stride-0 expanded) mask as int32, still a stride-0 expand where it was one
             m = torch.broadcast_to(mask if mask.dim() == len(shape) else mask.unsqueeze(-1), tuple(shape))
             if m.stride(-1) == 0:
                 mask = m[..., 0].to(torch.int32).contiguous().unsqueeze(-1).expand(tuple(shape))
@@ -376,7 +428,22 @@ class GaussianDiffusion:
                 mask = m.to(torch.int32).contiguous()
         if x_start is not None:
             x_start = x_start.to(torch.float32).contiguous()
-        x = x.to(torch.float32).contiguous()
+        return device, x.to(torch.float32).contiguous(), mask, x_start
+
+    def _loop(self, mode, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device, progress, top_p,
+              clamp_step, clamp_first, mask, x_start, eta, indices, want_aux):
+        """Generator of (sample, pred_xstart, mean, t) per reverse step.  Our denoiser, in-kernel noise, a [B, L, D] state
+        and `denoised_fn` either our rounding or None: the fused step bodies of `_fused_loop` (progressive loops, clamp
+        gating and `rounding_trace` included), replayed as captured CUDA graphs for chains of >= GRAPH_MIN_STEPS steps
+        unless `use_cuda_graph` is off or `ops.profile_step` is timing the launches.  What cannot be captured (arbitrary
+        `model` / `denoised_fn` callables, `noise_source`, other state shapes) runs step by step through `_step`; with our
+        denoiser there the posterior kernel also emits the bf16 operand of the next step's first GEMM, and the batch shares
+        one time-embedding row (all sequences share t inside the loops, diffusion.py:516,887)."""
+        device, x, mask, x_start = self._loop_inputs(model, shape, noise, device, mask, x_start)
+        fast = self._fast_model(model)
+        B = shape[0]
+        if len(indices) == 0:
+            return
         idx_list = list(indices)
         t_idx = torch.tensor(idx_list, dtype=torch.int32, device=device)
         t_model = self._model_timesteps(t_idx.long()).float()
@@ -544,6 +611,118 @@ class GaussianDiffusion:
                                              model_kwargs, device, progress, None, 0, True, mask, x_start, eta, indices,
                                              want_aux=True):
             yield {"sample": sample, "pred_xstart": pred}
+
+    # -------------------------------------------------------------------------------------- DPM-Solver++(2M)
+    def dpm_solver_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, model_kwargs=None,
+                               device=None, progress=False, mask=None, x_start=None, steps=20, t_start=None, order=2,
+                               only_last=False):
+        """DPM-Solver++(2M) (Lu et al., "DPM-Solver++", 2022, Algorithm 2; order=1 is its first-order form, DDIM at eta = 0):
+        `steps` model evaluations at the indices of `dpm_solver_indices` from `t_start` (default: the last index) down
+        to 0, starting from `noise` (the state at t_start; drawn like the other loops when None).  Each evaluation's x0 is
+        processed as in ddim_sample_loop (rounded when `denoised_fn` rounds, then clipped) and the last one is returned as
+        is.  The sampler draws no noise.  Not part of the reference, which samples with DDPM / DDIM only.  Returns the state
+        after every evaluation, the last being x0 (one element when only_last)."""
+        t_start = self.num_timesteps - 1 if t_start is None else int(t_start)
+        indices = dpm_solver_indices(self.alphas_cumprod, t_start, steps)
+        coef = dpm_solver_coefficients(self.alphas_cumprod, indices, order).astype(np.float32)
+        return _collect(self._dpm_loop(model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device, progress, mask,
+                                       x_start, indices, coef), only_last)
+
+    def _dpm_loop(self, model, shape, noise, clip_denoised, denoised_fn, model_kwargs, device, progress, mask, x_start, indices,
+                  coef):
+        """Generator of (state, None, None, t) per evaluation; path selection as in `_loop`: the fused body of
+        `_dpm_fused_loop` (graph-replayed for >= GRAPH_MIN_STEPS evaluations) or, for what cannot be captured, one
+        md_dpm_solver_step per evaluation with that evaluation's coefficient row."""
+        device, x, mask, x_start = self._loop_inputs(model, shape, noise, device, mask, x_start)
+        self._upload_schedule()
+        fast = self._fast_model(model)
+        B = shape[0]
+        t_idx = torch.tensor(indices, dtype=torch.int32, device=device)
+        t_model = self._model_timesteps(t_idx.long()).float()
+        coef = torch.from_numpy(coef).to(device)
+        ks = range(len(indices))
+        if progress:
+            from tqdm.auto import tqdm
+            ks = tqdm(ks)
+        E = rounding_weight_of(denoised_fn)
+        if fast is not None and self.noise_source is None and (E is not None or denoised_fn is None) and x.dim() == 3:
+            capture = self.use_cuda_graph and len(indices) >= self.GRAPH_MIN_STEPS and ops._PROFILE[0] is None
+            yield from self._dpm_fused_loop(fast, x, E, t_idx, t_model, coef, ks, clip_denoised, mask, x_start, capture)
+            return
+        hist = torch.empty_like(x)              # x0 of the previous evaluation (first-order rows never read it)
+        x_bf16 = None
+        for k in ks:
+            if fast is not None:
+                t_arg = t_idx[k:k + 1]
+                model_output = fast.denoise(x, t_model[k:k + 1], x_bf16=x_bf16, uniform_t=True)
+                Dp = fast.weight_pack().Dp
+                x_bf16 = (torch.empty_like(x, dtype=torch.bfloat16) if Dp == x.shape[-1]
+                          else torch.zeros(x.shape[:-1] + (Dp,), dtype=torch.bfloat16, device=x.device))
+            else:
+                t_arg = t_idx[k:k + 1].long().expand(B)
+                model_output = self._call_model(model, x, t_arg, model_kwargs)
+            E, idx, pred = self._processed_x0(x, t_arg, model_output, denoised_fn)
+            x = ops.dpm_solver_step(x, coef[k:k + 1], hist, idx=idx, pred=pred, E=E, mask=mask, x_start=x_start,
+                                    clip=clip_denoised, out_bf16=x_bf16)
+            yield x, None, None, t_arg
+
+    def _dpm_fused_loop(self, fast, x, E, t_idx, t_model, coef, ks, clip_denoised, mask, x_start, capture):
+        """`_fused_loop`'s structure with one body for every evaluation: md_step_advance -> denoiser (the last Linear emits
+        the split the rounding consumes) -> md_round_argmin_tc -> md_dpm_solver_step, which takes its coefficient row at the
+        cursor and updates x_t, its padded bf16 copy and the x0 history in place.  Everything the body touches is allocated
+        here, before the capture; the first evaluation runs eagerly, the second is captured and every later one replays it."""
+        dev = x.device
+        x = x.clone()
+        pk = fast.weight_pack()
+        xb = ops.cast_bf16(x, width=pk.Dp)
+        use_split = E is not None and self.predict_xstart and pk.has_down
+        mo = None if use_split else torch.empty_like(x)
+        mo_split = torch.empty(x.shape[:-1] + (2 * pk.Dp,), dtype=torch.bfloat16, device=dev) if use_split else None
+        cursor = torch.zeros(1, dtype=torch.int32, device=dev)
+        t_cur = torch.zeros(1, dtype=torch.int32, device=dev)
+        tm_cur = torch.zeros(1, dtype=torch.float32, device=dev)
+        ctr_cur = torch.zeros(1, dtype=torch.int64, device=dev)      # published by md_step_advance, unused: no noise
+        hist = torch.empty_like(x)
+        M = x.shape[0] * x.shape[1]
+        trace = self.rounding_trace if E is not None else None
+        idx = torch.empty((M,), dtype=torch.int32, device=dev) if E is not None else None
+        margin = torch.empty((M,), dtype=torch.float32, device=dev) if trace is not None else None
+        if E is not None:
+            se = ops.split_embedding(E)
+            E_step, clip_step = (se.E_clamped, 2) if clip_denoised else (E, 0)
+        post = dict(cursor=cursor, mask=mask, x_start=x_start, out=x, out_bf16=xb)
+
+        def model_x0():
+            out = fast.denoise(x, tm_cur, x_bf16=xb, uniform_t=True, out=mo)
+            return out if self.predict_xstart else ops.xstart_from_eps(x, out, t_cur)
+
+        def body():
+            ops.step_advance(cursor, t_idx, t_model, t_cur, tm_cur, ctr_cur, 0)
+            if E is None:
+                ops.dpm_solver_step(x, coef, hist, pred=model_x0(), clip=clip_denoised, **post)
+                return
+            if use_split:
+                fast.denoise(x, tm_cur, x_bf16=xb, uniform_t=True, split_out=mo_split)
+                ops.round_argmin_tc(None, se, out=idx, presplit=mo_split, margin_out=margin)
+            else:
+                ops.round_argmin_tc(model_x0(), se, out=idx, margin_out=margin)
+            ops.dpm_solver_step(x, coef, hist, idx=idx, E=E_step, clip=clip_step, **post)
+
+        graph, nodes = None, 0
+        for k in ks:
+            if k == 0 or not capture:
+                body()
+            else:
+                if graph is None:
+                    before = ops.launch_count()
+                    graph = _capture(dev, body)
+                    nodes = ops.launch_count() - before          # kernels recorded by the capture (nothing ran yet)
+                    ops.add_launches(-nodes)
+                graph.replay()
+                ops.add_launches(nodes)
+            if trace is not None:
+                trace.append((idx.clone(), margin.clone()))
+            yield x, None, None, t_idx[k:k + 1]
 
 
 class SpacedDiffusion(GaussianDiffusion):

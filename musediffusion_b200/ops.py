@@ -359,6 +359,35 @@ def posterior_step(x_t, t, mode, idx=None, pred=None, E=None, noise=None, seed=0
     return out
 
 
+def dpm_solver_step(x_t, coef, pred_hist, idx=None, pred=None, E=None, cursor=None, mask=None, x_start=None, clip=True, out=None,
+                    out_bf16=None):
+    """One DPM-Solver++(2M) update (md_dpm_solver_step).  coef: fp32 [n, 4] rows (a, b, c0, c1); without `cursor` it has one
+    row, with it the kernel takes row *cursor - 1.  pred_hist: fp32 [B, L, D], read where c1 != 0 and overwritten with this
+    step's processed x0.  `out` may be x_t itself.  clip and out_bf16 as in posterior_step."""
+    x_t = _c(x_t, torch.float32)
+    B, L, D = x_t.shape
+    keep, mask_t, ts, ds = _mask_args(mask, B, L, D)
+    if out is None:
+        out = torch.empty_like(x_t)
+    if pred is not None:
+        pred = _c(pred, torch.float32)
+    if idx is not None:
+        idx = _c(idx, torch.int32)
+    if x_start is not None:
+        x_start = _c(x_start, torch.float32)
+    if (idx is None) == (pred is None):
+        raise _lib.MuseDiffLibraryError("md_dpm_solver_step: exactly one of idx / pred_in")
+    if coef.dtype != torch.float32 or coef.dim() != 2 or coef.shape[1] != 4 or not coef.is_contiguous():
+        raise _lib.MuseDiffLibraryError("md_dpm_solver_step: coef must be a contiguous fp32 [n, 4] table")
+    if pred_hist.dtype != torch.float32 or pred_hist.shape != x_t.shape or not pred_hist.is_contiguous():
+        raise _lib.MuseDiffLibraryError("md_dpm_solver_step: pred_hist must be a contiguous fp32 tensor shaped like x_t")
+    if cursor is not None and (cursor.dtype != torch.int32 or cursor.numel() != 1):
+        raise _lib.MuseDiffLibraryError("md_dpm_solver_step: cursor must be one int32")
+    _cu(x_t, idx, pred, E, pred_hist, coef, cursor, mask_t, x_start, out, out_bf16)
+    K.dpm_solver_step(x_t, idx, pred, E, pred_hist, coef, cursor, mask_t, ts, ds, x_start, out, out_bf16, int(clip))
+    return out
+
+
 def xstart_from_eps(x_t, eps, t):
     x_t = _c(x_t, torch.float32)
     eps = _c(eps, torch.float32)

@@ -29,12 +29,23 @@ def build_model_emb(model, device):
     return emb
 
 
+SAMPLERS = ("reference", "dpm_solver++")
+
+
 @torch.no_grad()
 def sample_batch(model, diffusion, model_emb, cond, mode, step, diffusion_steps, strength=0.75, top_p=1, clamp_step=0,
-                 clip_denoised=True, device=None, fused_decode=True, return_sample=False):
+                 clip_denoised=True, device=None, fused_decode=True, return_sample=False, sampler="reference"):
     """run/sample.py:177-220 for one batch: cond = {'input_ids', 'input_mask'} (host or device int tensors) ->
     int64 token ids [B, L] on the device.  `fused_decode=False` keeps the reference's get_logits + argmax pair;
-    `return_sample=True` also returns the final x_0 estimate `samples[-1]` (fp32 [B, L, D])."""
+    `return_sample=True` also returns the final x_0 estimate `samples[-1]` (fp32 [B, L, D]).
+    `sampler="dpm_solver++"` (not in the reference) samples with `diffusion.dpm_solver_sample_loop` in `step` model
+    evaluations instead of the reference's DDPM / DDIM choice; top_p and clamp_step do not apply to it.  Its modification
+    mode starts at index t_start = int(strength * T) - 1 of the diffusion's T indices, so `strength` is the fraction of the
+    chain whatever `step` is (the reference's DDIM starts at int(step * strength) - 1 and reads the table with gap
+    T // step)."""
+    if sampler not in SAMPLERS:
+        raise ValueError("sampler must be one of %s, got %r" % (SAMPLERS, sampler))
+    dpm = sampler == "dpm_solver++"
     device = device or next(model.parameters()).device
     input_ids = torch.as_tensor(cond["input_ids"]).to(device, non_blocking=True)
     mask_ori = torch.as_tensor(cond["input_mask"]).to(device, non_blocking=True)
@@ -42,6 +53,7 @@ def sample_batch(model, diffusion, model_emb, cond, mode, step, diffusion_steps,
     input_ids_mask = torch.broadcast_to(mask_ori.unsqueeze(dim=-1), x_start.shape)      # :186
     if mode == "generation":                                                            # :190-193
         noising_t = None
+        t_start = diffusion.num_timesteps - 1
         if diffusion.noise_source is not None:
             noise = diffusion._external_noise(x_start.shape, "randn", device)
         else:
@@ -50,16 +62,25 @@ def sample_batch(model, diffusion, model_emb, cond, mode, step, diffusion_steps,
                                 step_counter=diffusion._next_counter(), seq_offset=diffusion.seq_offset, mask=mask_ori)
     else:                                                                               # :195-197
         noising_t = int(step * strength)
-        timestep = torch.full((x_start.shape[0], 1), noising_t - 1, device=device)
+        t_start = int(strength * diffusion.num_timesteps) - 1 if dpm else noising_t - 1
+        if dpm and t_start < 0:
+            raise ValueError("strength=%r leaves no diffusion index to start from (T=%d)" % (strength, diffusion.num_timesteps))
+        timestep = torch.full((x_start.shape[0], 1), t_start, device=device)
         x_noised = diffusion.q_sample(x_start.unsqueeze(-1), timestep, mask=input_ids_mask).squeeze(-1)
-    if step == diffusion_steps:                                                         # :109-114
-        gap, sample_fn = 1, diffusion.p_sample_loop
+    denoised_fn = partial(denoised_fn_round, model_emb, dist=None)
+    if dpm:
+        samples = diffusion.dpm_solver_sample_loop(model=model, shape=tuple(x_start.shape), noise=x_noised,
+                                                   clip_denoised=clip_denoised, denoised_fn=denoised_fn, model_kwargs=cond,
+                                                   mask=input_ids_mask, x_start=x_start, steps=step, t_start=t_start,
+                                                   only_last=True)
     else:
-        gap, sample_fn = diffusion_steps // step, diffusion.ddim_sample_loop
-    samples = sample_fn(model=model, shape=tuple(x_start.shape), noise=x_noised, clip_denoised=clip_denoised,
-                        denoised_fn=partial(denoised_fn_round, model_emb, dist=None), model_kwargs=cond, top_p=top_p,
-                        clamp_step=clamp_step, clamp_first=True, mask=input_ids_mask, x_start=x_start, gap=gap,
-                        t_enc=noising_t, only_last=True)                                # :200-215
+        if step == diffusion_steps:                                                     # :109-114
+            gap, sample_fn = 1, diffusion.p_sample_loop
+        else:
+            gap, sample_fn = diffusion_steps // step, diffusion.ddim_sample_loop
+        samples = sample_fn(model=model, shape=tuple(x_start.shape), noise=x_noised, clip_denoised=clip_denoised,
+                            denoised_fn=denoised_fn, model_kwargs=cond, top_p=top_p, clamp_step=clamp_step, clamp_first=True,
+                            mask=input_ids_mask, x_start=x_start, gap=gap, t_enc=noising_t, only_last=True)   # :200-215
     sample = samples[-1]
     if fused_decode:
         tokens = model.decode_tokens(sample)
@@ -116,6 +137,9 @@ def create_parser():
         sp.add_argument("--clamp_step", type=int, default=0)
         sp.add_argument("--sample_seed", type=int, default=105)
         sp.add_argument("--clip_denoised", type=lambda s: s.lower() in ("1", "true", "yes"), default=True)
+        sp.add_argument("--sampler", choices=SAMPLERS, default="reference",
+                        help="reference: the reference's DDPM (--step = diffusion_steps) or DDIM; dpm_solver++: DPM-Solver++(2M) "
+                             "with --step model evaluations (not in the reference; --strength is then the fraction of the chain)")
         sp.add_argument("--input_npz", default=None, help="npz with input_ids/input_mask [N, L] (else synthetic)")
         sp.add_argument("--strict_validation", action="store_true",
                         help="also run validate_rigidly (the reference does when it computes metrics, run/sample.py:240)")
@@ -241,7 +265,7 @@ def main(argv=None):
             cond = {"input_ids": torch.from_numpy(ids_all[sl]), "input_mask": torch.from_numpy(mask_all[sl])}
             tok = sample_batch(model, diffusion, model_emb, cond, args.mode, args.step, targs.diffusion_steps,
                                strength=getattr(args, "strength", 0.75), top_p=args.top_p, clamp_step=args.clamp_step,
-                               clip_denoised=args.clip_denoised, device=dev)
+                               clip_denoised=args.clip_denoised, device=dev, sampler=args.sampler)
             tok_pad[:tok.shape[0]] = tok.to(torch.int32)
         # decoded ids of the round to every rank with ONE NCCL all-gather ([world, batch, L] int32), instead of the reference's
         # rank-after-rank decode with a broadcast + barrier per rank (run/sample.py:222-294)
